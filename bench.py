@@ -14,6 +14,9 @@ A STEP is one batch of FRAMES_PER_STEP frames through one session (one session p
 
 `--impl reference` times the CPU path only (the reference's own videoconvert+x264enc pipeline cannot
 run here — SURVEY.md §8c — so the arm runs the oracle port, all host threads, labelled kind="port").
+
+`--dump-outputs DIR` writes what the `value` leg delivered in its last timed step (64 access units and their frame fields) as .npy
+files; the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -380,6 +383,26 @@ def emit(line: dict):
     os.write(_REAL_STDOUT if _REAL_STDOUT is not None else 1, data)
 
 
+DUMP_BYTES_MAX = 64 << 20
+
+
+def dump_outputs(out_dir: str, frames: list) -> None:
+    """`frames`: (frame_id, is_key, qp, pts90k, access unit) per picture, in delivery order — what the callback of the timed path
+    receives.  The per-picture fields go to one float64 array each, the access units, concatenated, to access_unit_bytes.npy as
+    float32; beyond DUMP_BYTES_MAX in all, a fixed seeded sample of byte positions is kept, with the positions."""
+    os.makedirs(out_dir, exist_ok=True)
+    meta = np.array([f[:4] + (len(f[4]),) for f in frames], np.float64)
+    for i, name in enumerate(("frame_id", "is_key", "qp", "pts90k", "access_unit_size")):
+        np.save(os.path.join(out_dir, name + ".npy"), meta[:, i])
+    data = np.frombuffer(b"".join(f[4] for f in frames), np.uint8)
+    budget = (DUMP_BYTES_MAX - meta.nbytes - 4096) // 4          # 4096: the .npy headers
+    if data.size > budget:
+        pos = np.sort(np.random.default_rng(0).choice(data.size, budget // 3, replace=False))   # float32 byte + float64 position
+        np.save(os.path.join(out_dir, "access_unit_byte_positions.npy"), pos.astype(np.float64))
+        data = data[pos]
+    np.save(os.path.join(out_dir, "access_unit_bytes.npy"), data.astype(np.float32))
+
+
 def main():
     own_stdout()
     ap = argparse.ArgumentParser()
@@ -388,7 +411,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the access units of the last timed step (rank 0) to DIR/*.npy, to compare two builds output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's output; --impl reference has none")
     if args.warmup < 3:
         args.warmup = 3
     rank = int(os.environ.get("RANK", "0"))
@@ -453,11 +480,19 @@ def main():
                    ring_slots=N_DISTINCT, flags=0, collect=False)
     out_bytes = [0]
     sample_aus = []
+    # --dump-outputs: the access units of the last timed step of leg 1, picked by frame id (16 bits on the wire, hence the mask);
+    # the later legs on this session continue the ids, so the capture stops after one step
+    dump_first = (args.warmup + args.steps - 1) * FRAMES_PER_STEP if args.dump_outputs and rank == 0 else None
+    last_step = []
 
     def on_frame(fptr):
         out_bytes[0] += fptr.contents.size
         if len(sample_aus) < 8 and not fptr.contents.is_key:
             sample_aus.append(ctypes.string_at(fptr.contents.data, fptr.contents.size))
+        if dump_first is not None and len(last_step) < FRAMES_PER_STEP:
+            f = fptr.contents
+            if (f.frame_id - dump_first) & 0xFFFF < FRAMES_PER_STEP:
+                last_step.append((f.frame_id, f.is_key, f.qp, f.pts90k, ctypes.string_at(f.data, f.size)))
     sess._on_frame = on_frame
 
     # ---------------- leg 1: inputs resident in HBM ----------------------------------------------------
@@ -743,6 +778,9 @@ def main():
             cpu = {"value": None, "error": repr(e)}
 
     if rank == 0:
+        if dump_first is not None:
+            assert len(last_step) == FRAMES_PER_STEP, f"{len(last_step)} of the last step's {FRAMES_PER_STEP} access units captured"
+            dump_outputs(args.dump_outputs, last_step)
         line = {
             "metric": "4K frames/sec encoded", "value": value, "unit": "frames/s", "n_gpus": world, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": t_ms / args.steps, "higher_is_better": True, "scaling": "weak",
