@@ -188,8 +188,6 @@ int  b2v_bench_csc_burst(void* h, int32_t n_resident, int32_t iters, float* ms_p
  * stop = after every frame submitted since has been delivered.  bench.py times its K steps with it. */
 int  b2v_timer_start(void* h);
 int  b2v_timer_stop(void* h, float* ms);
-/* launch-shape tuning hook for the CSC fast path (tools/csc_sweep.py): units per thread, block size, grid.y (0 = auto) */
-void b2v_tune_csc(int units_per_thread, int block, int grid_y);
 const char* b2v_last_error(void);
 
 /* ---- RTP H.264 payloader (SURVEY.md §8f row 1): replaces H264Encoder.pack -> _split_bitstream / _packetize

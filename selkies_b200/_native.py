@@ -86,7 +86,6 @@ SYMBOLS = [
     ("b2v_bench_csc_burst", C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_float)]),
     ("b2v_timer_start", C.c_int, [C.c_void_p]),
     ("b2v_timer_stop", C.c_int, [C.c_void_p, C.POINTER(C.c_float)]),
-    ("b2v_tune_csc", None, [C.c_int, C.c_int, C.c_int]),
     ("b2v_last_error", C.c_char_p, []),
     ("b2v_rtp_h264_packetize", C.c_int, [C.c_char_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int32,
                                          C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int32)]),

@@ -98,10 +98,8 @@ struct Session {
   cudaEvent_t ev_h2d[kMaxSlots] = {}, ev_csc[kMaxSlots] = {};
   uint8_t slot_state[kMaxSlots] = {};   // SLOT_*
   size_t frame_bytes = 0;
-  void* tmap_slot[kMaxSlots] = {};       // device-resident tensor maps of dev_slot[] (TMA CSC path; null = LDG kernel)
   // resident frames (bench `value` leg)
   std::vector<uint8_t*> resident;
-  std::vector<void*> tmap_res;
   // scaling taps
   Tap *d_tx = nullptr, *d_ty = nullptr;
   // current-frame NV12 (coded size)
@@ -156,7 +154,6 @@ int alloc_geometry(Session* s) {
   for (int i = 0; i < s->n_slots; i++) {
     CK(cudaHostAlloc((void**)&s->host_slot[i], s->frame_bytes, cudaHostAllocDefault));
     CK(cudaMalloc((void**)&s->dev_slot[i], s->frame_bytes));
-    s->tmap_slot[i] = (s->dst_w == s->src_w && s->dst_h == s->src_h) ? csc_make_tensor_map(s->dev_slot[i], s->src_w, s->src_h, s->src_w * 4) : nullptr;
     s->slot_state[i] = SLOT_FREE;
   }
   CK(cudaMalloc((void**)&s->d_cur, (size_t)s->coded_w * s->coded_h * 3 / 2));
@@ -211,12 +208,10 @@ void free_geometry(Session* s) {
     if (s->dev_slot[i]) cudaFree(s->dev_slot[i]);
     if (s->d_au[i]) cudaFree(s->d_au[i]);
     if (s->h_out[i]) cudaFreeHost(s->h_out[i]);
-    csc_free_tensor_map(s->tmap_slot[i]);
-    s->host_slot[i] = s->dev_slot[i] = s->d_au[i] = s->h_out[i] = nullptr; s->tmap_slot[i] = nullptr;
+    s->host_slot[i] = s->dev_slot[i] = s->d_au[i] = s->h_out[i] = nullptr;
   }
   for (auto p : s->resident) if (p) cudaFree(p);
-  for (auto p : s->tmap_res) csc_free_tensor_map(p);
-  s->resident.clear(); s->tmap_res.clear();
+  s->resident.clear();
   if (s->d_cur) cudaFree(s->d_cur);
   if (s->d_tx) cudaFree(s->d_tx);
   if (s->d_ty) cudaFree(s->d_ty);
@@ -225,9 +220,8 @@ void free_geometry(Session* s) {
   if (s->jenc) { jpeg_destroy(s->jenc); s->jenc = nullptr; }
 }
 
-CscParams csc_params(Session* s, const uint8_t* d_bgra, int stride, uint8_t* d_nv12, const void* tmap = nullptr) {
+CscParams csc_params(Session* s, const uint8_t* d_bgra, int stride, uint8_t* d_nv12) {
   CscParams p{};
-  p.tmap = stride == s->src_w * 4 ? tmap : nullptr;
   p.src = d_bgra; p.src_w = s->src_w; p.src_h = s->src_h; p.src_stride = stride;
   p.dst_w = s->dst_w; p.dst_h = s->dst_h; p.coded_w = s->coded_w; p.coded_h = s->coded_h;
   p.out_y = d_nv12; p.out_uv = d_nv12 + (size_t)s->coded_w * s->coded_h;
@@ -395,7 +389,7 @@ int submit_failed(Session* s, int out_idx, int in_slot, cudaError_t e, const cha
   do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return submit_failed(s, out_idx, in_slot, e_, #call); } while (0)
 
 // common tail of b2v_ring_submit / b2v_submit_resident: CSC + encode + D2H + job
-int submit_common(Session* s, const uint8_t* d_bgra, int stride, int in_slot, int64_t capture_ns, const void* tmap) {
+int submit_common(Session* s, const uint8_t* d_bgra, int stride, int in_slot, int64_t capture_ns) {
   int out_idx = 0;
   Job j{};
   EncodeFrameParams fp{};
@@ -437,7 +431,7 @@ int submit_common(Session* s, const uint8_t* d_bgra, int stride, int in_slot, in
     s->submitted++;
     s->stats.frames_submitted++;
   }
-  CscParams cp = csc_params(s, d_bgra, stride, s->d_cur, tmap);
+  CscParams cp = csc_params(s, d_bgra, stride, s->d_cur);
   cudaEvent_t* ev = j.timing ? s->ev_t[out_idx] : nullptr;
   if (ev && s->d_csc_ts && s->encode) {
     cp.ts = s->d_csc_ts + 2 * out_idx;
@@ -445,7 +439,7 @@ int submit_common(Session* s, const uint8_t* d_bgra, int stride, int in_slot, in
     cudaMemsetAsync(cp.ts + 1, 0, sizeof(unsigned long long), s->st_enc);
   }
   if (ev) cudaEventRecord(ev[0], s->st_enc);
-  int nl = launch_csc(cp, s->sm_count, s->st_enc);
+  int nl = launch_csc(cp, s->st_enc);
   if (ev) cudaEventRecord(ev[1], s->st_enc);
   if (in_slot >= 0) CKS(cudaEventRecord(s->ev_csc[in_slot], s->st_enc));
   CKS(cudaEventRecord(s->ev_enc[out_idx], s->st_enc));
@@ -635,7 +629,7 @@ int b2v_ring_submit(void* h, int32_t slot, int32_t stride, int64_t capture_ns) {
     s->stats.h2d_bytes += (int64_t)stride * s->src_h;
     s->stats.ns_submit += now_ns() - t0;
   }
-  return submit_common(s, s->dev_slot[slot], stride, slot, capture_ns, s->tmap_slot[slot]);
+  return submit_common(s, s->dev_slot[slot], stride, slot, capture_ns);
 }
 
 int b2v_resident_upload(void* h, int32_t index, const void* bgra, int32_t stride) {
@@ -644,11 +638,8 @@ int b2v_resident_upload(void* h, int32_t index, const void* bgra, int32_t stride
   if (stride <= 0) stride = s->src_w * 4;
   std::lock_guard<std::mutex> sub(s->submit_mu);
   CK(cudaSetDevice(s->device));
-  if ((int)s->resident.size() <= index) { s->resident.resize(index + 1, nullptr); s->tmap_res.resize(index + 1, nullptr); }
-  if (!s->resident[index]) {
-    CK(cudaMalloc((void**)&s->resident[index], s->frame_bytes));
-    if (s->dst_w == s->src_w && s->dst_h == s->src_h) s->tmap_res[index] = csc_make_tensor_map(s->resident[index], s->src_w, s->src_h, s->src_w * 4);
-  }
+  if ((int)s->resident.size() <= index) s->resident.resize(index + 1, nullptr);
+  if (!s->resident[index]) CK(cudaMalloc((void**)&s->resident[index], s->frame_bytes));
   CK(cudaMemcpy2D(s->resident[index], (size_t)s->src_w * 4, bgra, stride, (size_t)s->src_w * 4, s->src_h, cudaMemcpyHostToDevice));
   return 0;
 }
@@ -658,7 +649,7 @@ int b2v_submit_resident(void* h, int32_t index, int64_t capture_ns) {
   if (!s || index < 0 || index >= (int)s->resident.size() || !s->resident[index]) return fail(B2V_EINVAL, "resident frame %d not uploaded", index);
   std::lock_guard<std::mutex> sub(s->submit_mu);
   CK(cudaSetDevice(s->device));
-  return submit_common(s, s->resident[index], s->src_w * 4, -1, capture_ns, s->tmap_res[index]);
+  return submit_common(s, s->resident[index], s->src_w * 4, -1, capture_ns);
 }
 
 int b2v_flush(void* h) {
@@ -776,14 +767,13 @@ int b2v_csc_nv12(void* h, const void* bgra, int32_t stride, void* nv12) {
   CK(cudaMalloc((void**)&d_in, (size_t)s->src_w * 4 * s->src_h));
   CK(cudaMalloc((void**)&d_out, out_bytes));
   CK(cudaMemcpy2DAsync(d_in, (size_t)s->src_w * 4, bgra, stride, (size_t)s->src_w * 4, s->src_h, cudaMemcpyHostToDevice, s->st_enc));
-  void* tm = (s->dst_w == s->src_w && s->dst_h == s->src_h) ? csc_make_tensor_map(d_in, s->src_w, s->src_h, s->src_w * 4) : nullptr;
-  CscParams p = csc_params(s, d_in, s->src_w * 4, d_out, tm);
+  CscParams p = csc_params(s, d_in, s->src_w * 4, d_out);
   p.coded_w = s->dst_w; p.coded_h = s->dst_h;          // visible region only
   p.out_uv = d_out + (size_t)s->dst_w * s->dst_h;
-  launch_csc(p, s->sm_count, s->st_enc);
+  launch_csc(p, s->st_enc);
   CK(cudaMemcpyAsync(nv12, d_out, out_bytes, cudaMemcpyDeviceToHost, s->st_enc));
   CK(cudaStreamSynchronize(s->st_enc));
-  cudaFree(d_in); cudaFree(d_out); csc_free_tensor_map(tm);
+  cudaFree(d_in); cudaFree(d_out);
   CK(cudaGetLastError());
   return 0;
 }
@@ -813,8 +803,8 @@ int b2v_bench_csc(void* h, int32_t n_resident, int32_t iters, float* ms_per_laun
   size_t ob = (size_t)s->coded_w * s->coded_h * 3 / 2;
   for (auto& o : outs) CK(cudaMalloc((void**)&o, ob));
   for (int i = 0; i < n_resident; i++) {   // warm-up: one pass over every frame
-    CscParams p = csc_params(s, s->resident[i], s->src_w * 4, outs[i], s->tmap_res[i]);
-    launch_csc(p, s->sm_count, s->st_enc);
+    CscParams p = csc_params(s, s->resident[i], s->src_w * 4, outs[i]);
+    launch_csc(p, s->st_enc);
   }
   CK(cudaStreamSynchronize(s->st_enc));
   // each launch is bracketed by its own event pair; the sum excludes host launch gaps
@@ -822,9 +812,9 @@ int b2v_bench_csc(void* h, int32_t n_resident, int32_t iters, float* ms_per_laun
   for (int i = 0; i < iters; i++) { cudaEventCreate(&e0[i]); cudaEventCreate(&e1[i]); }
   for (int i = 0; i < iters; i++) {
     int k = i % n_resident;
-    CscParams p = csc_params(s, s->resident[k], s->src_w * 4, outs[k], s->tmap_res[k]);
+    CscParams p = csc_params(s, s->resident[k], s->src_w * 4, outs[k]);
     cudaEventRecord(e0[i], s->st_enc);
-    launch_csc(p, s->sm_count, s->st_enc);
+    launch_csc(p, s->st_enc);
     cudaEventRecord(e1[i], s->st_enc);
   }
   CK(cudaStreamSynchronize(s->st_enc));
@@ -871,11 +861,11 @@ int b2v_bench_csc_burst(void* h, int32_t n_resident, int32_t iters, float* ms_pe
   std::vector<uint8_t*> outs(n_resident, nullptr);
   size_t ob = (size_t)s->coded_w * s->coded_h * 3 / 2;
   for (auto& o : outs) CK(cudaMalloc((void**)&o, ob));
-  for (int i = 0; i < n_resident; i++) launch_csc(csc_params(s, s->resident[i], s->src_w * 4, outs[i], s->tmap_res[i]), s->sm_count, s->st_enc);
+  for (int i = 0; i < n_resident; i++) launch_csc(csc_params(s, s->resident[i], s->src_w * 4, outs[i]), s->st_enc);
   CK(cudaStreamSynchronize(s->st_enc));
   cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
   cudaEventRecord(e0, s->st_enc);
-  for (int i = 0; i < iters; i++) { int k = i % n_resident; launch_csc(csc_params(s, s->resident[k], s->src_w * 4, outs[k], s->tmap_res[k]), s->sm_count, s->st_enc); }
+  for (int i = 0; i < iters; i++) { int k = i % n_resident; launch_csc(csc_params(s, s->resident[k], s->src_w * 4, outs[k]), s->st_enc); }
   cudaEventRecord(e1, s->st_enc);
   CK(cudaStreamSynchronize(s->st_enc));
   float ms = 0; cudaEventElapsedTime(&ms, e0, e1);

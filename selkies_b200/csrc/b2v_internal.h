@@ -23,16 +23,11 @@ struct CscParams {
   const Tap* tx;        // dst_w taps (null when 1:1)
   const Tap* ty;        // dst_h taps
   unsigned long long* ts; // null, or {min block-start, max block-end} %globaltimer stamps of this launch (B2V_FLAG_TIMING)
-  const void* tmap;       // null, or the device-resident CUtensorMap of `src` (csc_make_tensor_map): enables the TMA kernel
   int matrix;             // 0 = BT.709 limited range (H.264 path), 1 = JFIF full-range BT.601 (JPEG stripe path)
 };
 
 // returns number of kernel launches issued (1)
-int launch_csc(const CscParams& p, int sm_count, cudaStream_t st);
+int launch_csc(const CscParams& p, cudaStream_t st);
 void make_taps_host(Tap* t, int dn, int sn);
-// 2-D tensor map of one BGRA source buffer for the TMA path, in device memory; null when the buffer does not qualify (the LDG
-// kernel is used then).  Owned by the caller: csc_free_tensor_map.
-void* csc_make_tensor_map(const uint8_t* d_bgra, int w, int h, int stride);
-void csc_free_tensor_map(void* tmap);
 
 }  // namespace b2v

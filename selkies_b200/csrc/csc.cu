@@ -8,21 +8,15 @@
 // Roofline: HBM-bound streaming kernel, 4 B/px read + 1.5 B/px written (5.5 B/px algorithmic).
 //   fast path  (1:1, width % 4 == 0): one thread = 4 px x 2 rows per unit: two 16-byte loads
 //              (ld.global.nc.L1::no_allocate.v4), two 4-byte Y stores and one 4-byte CbCr store, all
-//              warp-contiguous (512 B / 128 B / 128 B per warp instruction).  U units per thread are
-//              issued back to back so 2U 16-byte loads are in flight per thread.
+//              warp-contiguous (512 B / 128 B / 128 B per warp instruction).  Two units per thread are
+//              issued back to back so four 16-byte loads are in flight per thread.
 //   arithmetic: dp2a (two 16-bit coefficient x 8-bit pixel MACs per instruction); rounding
 //              constant and the +16 / +128 offsets are folded into the accumulator seed.
-//   TMA path   (1:1, the default on sm_100a): persistent grid of 2 CTAs per SM; one elected thread streams 256 px x 16 row
-//              BGRA tiles (16 KB) into a 4-stage shared-memory ring with cp.async.bulk.tensor.2d (SASS: UTMALDG) completing on
-//              mbarriers, so 128 KB of reads per SM are in flight with no load instruction in the compute warps' issue slots;
-//              the 256 threads convert from shared memory (conflict-free LDS.128) and store Y/CbCr straight to HBM.
-//   general path (scaled or ragged widths): one thread per 2x2 output block, taps from tables.
-#include <cuda.h>
-
-#include <cstdlib>
-#include <cstring>
-#include <mutex>
-
+//   scaled path (bilinear scale, 16-byte aligned source): one CTA per 64 x 8 output tile, its source footprint staged in
+//              shared memory.
+//   general path (ragged widths, unaligned scaled sources, footprints over 96 KB): one thread per 2x2 output block, taps
+//              from tables.
+// A TMA / mbarrier variant of the 1:1 kernel was built, measured slower at 4K and equal at 8K, and removed (profiles/README.md).
 #include "b2v_internal.h"
 
 namespace b2v {
@@ -31,11 +25,9 @@ namespace b2v {
 #ifdef CSC_TRACE
 __device__ __forceinline__ unsigned long long trace_now() { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; }
 #define TRACE_START(cta) do { if (threadIdx.x == 0) { unsigned sm; asm volatile("mov.u32 %0, %%smid;" : "=r"(sm)); g_trace[4 * (cta)] = trace_now(); g_trace[4 * (cta) + 2] = sm; } } while (0)
-#define TRACE_DATA(cta) do { if (threadIdx.x == 0) g_trace[4 * (cta) + 3] = trace_now(); } while (0)
 #define TRACE_END(cta) do { __syncthreads(); if (threadIdx.x == 0) g_trace[4 * (cta) + 1] = trace_now(); } while (0)
 #else
 #define TRACE_START(cta)
-#define TRACE_DATA(cta)
 #define TRACE_END(cta)
 #endif
 
@@ -50,17 +42,6 @@ __device__ __forceinline__ uint4 ld_stream(const uint8_t* p) {
   asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];"
                : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
   return v;
-}
-// same load with an L2 evict-first policy: the BGRA input is read exactly once, so it should be the first thing L2 drops — the
-// encoder's working set (reconstruction, NV12 source, coefficients) stays resident between its kernels
-__device__ __forceinline__ uint4 ld_stream_ef(const uint8_t* p, unsigned long long pol) {
-  uint4 v;
-  asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v4.u32 {%0,%1,%2,%3}, [%4], %5;"
-               : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p), "l"(pol));
-  return v;
-}
-__device__ __forceinline__ unsigned long long policy_evict_first() {
-  unsigned long long pol; asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol)); return pol;
 }
 __device__ __forceinline__ void st_stream(uint8_t* p, unsigned v) {
   asm volatile("st.global.cs.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
@@ -118,10 +99,12 @@ __device__ __forceinline__ void convert_quad(const uint4& a, const uint4& b, uns
 
 // ---- fast path ---------------------------------------------------------------------------
 // grid.x covers 4-px quads of a row, grid.y strides over groups of U row pairs.
-template <int U, bool EF, int M = 0>
+constexpr int CSC_U = 2;         // units (row pairs) per thread
+constexpr int CSC_BLOCK = 160;   // threads per block (launch_csc steps down to 128 / 96 / 64 when one of those divides the row)
+template <int M>
 __global__ void __launch_bounds__(256) csc_bgra_nv12_fast(CscParams p, int quads, int pairs) {
+  constexpr int U = CSC_U;
   const int q = blockIdx.x * blockDim.x + threadIdx.x;
-  const unsigned long long pol = EF ? policy_evict_first() : 0ull;
   TRACE_START(blockIdx.y * gridDim.x + blockIdx.x);
   if (p.ts && threadIdx.x == 0) {   // device-side stopwatch of this launch: first block start .. last block end
     unsigned long long t0; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0)); atomicMin(p.ts, t0);
@@ -135,8 +118,8 @@ __global__ void __launch_bounds__(256) csc_bgra_nv12_fast(CscParams p, int quads
       int pr = pr0 + u;
       if (pr < pairs) {
         int r0 = min(2 * pr, p.src_h - 1), r1 = min(2 * pr + 1, p.src_h - 1);   // bottom padding rows replicate
-        a[u] = EF ? ld_stream_ef(src + (size_t)r0 * p.src_stride, pol) : ld_stream(src + (size_t)r0 * p.src_stride);
-        b[u] = EF ? ld_stream_ef(src + (size_t)r1 * p.src_stride, pol) : ld_stream(src + (size_t)r1 * p.src_stride);
+        a[u] = ld_stream(src + (size_t)r0 * p.src_stride);
+        b[u] = ld_stream(src + (size_t)r1 * p.src_stride);
       }
     }
 #pragma unroll
@@ -156,123 +139,6 @@ __global__ void __launch_bounds__(256) csc_bgra_nv12_fast(CscParams p, int quads
     if (threadIdx.x == 0) { unsigned long long t1; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1)); atomicMax(p.ts + 1, t1); }
   }
   TRACE_END(blockIdx.y * gridDim.x + blockIdx.x);
-}
-
-// ---- TMA path --------------------------------------------------------------------------------------------------------------
-// Persistent and warp-specialised: gridDim.x CTAs (a few per SM) walk the tile list t = blockIdx.x, + gridDim.x, ...
-// Tile = 256 px x 16 rows of BGRA = 16 KB.  The PRODUCER warp's elected lane fetches each tile with ONE
-// cp.async.bulk.tensor.2d (SASS: UTMALDG) into stage k % STAGES of a shared-memory ring; the bytes landing complete the stage's
-// `full` mbarrier.  Eight CONSUMER warps each own one row pair of the tile (2 x 256 px: two 4x2 units per lane, conflict-free
-// LDS.128), convert, store Y / CbCr straight to global memory and arrive on the stage's `empty` mbarrier, which lets the
-// producer refill it — no block-wide barrier anywhere, the warps drift apart and overlap each other's latencies.
-// Rows / columns beyond the picture are zero-filled by the TMA unit (their stores are guarded).
-constexpr int TMA_TW = 256, TMA_TH = 16;
-constexpr int TMA_TILE_BYTES = TMA_TW * 4 * TMA_TH;
-constexpr int TMA_CONSUMER_WARPS = TMA_TH / 2;
-constexpr int TMA_THREADS = 32 * (TMA_CONSUMER_WARPS + 1);
-constexpr int TMA_MAX_STAGES = 6;
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "WAIT_%=:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra DONE_%=;\n"
-      "bra WAIT_%=;\n"
-      "DONE_%=:\n"
-      "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void tma_load_2d(void* dst, const void* map, int x, int y, uint64_t* bar) {
-  asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-               ::"r"(smem_u32(dst)), "l"(map), "r"(x), "r"(y), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ uint4 lds128(const uint8_t* p) {
-  uint4 v;
-  asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(smem_u32(p)));
-  return v;
-}
-__device__ __forceinline__ void st_y_uv(const CscParams& p, int x, int pr, unsigned y0, unsigned y1, unsigned uv) {
-  *reinterpret_cast<unsigned*>(p.out_y + (size_t)(2 * pr) * p.coded_w + x) = y0;
-  *reinterpret_cast<unsigned*>(p.out_y + (size_t)(2 * pr + 1) * p.coded_w + x) = y1;
-  *reinterpret_cast<unsigned*>(p.out_uv + (size_t)pr * p.coded_w + x) = uv;
-}
-
-__global__ void __launch_bounds__(TMA_THREADS)
-csc_bgra_nv12_tma(CscParams p, int tiles_x, int n_tiles, int stages) {
-  extern __shared__ __align__(128) uint8_t tma_smem[];            // stages x 16 KB
-  __shared__ __align__(8) uint64_t full[TMA_MAX_STAGES], empty[TMA_MAX_STAGES];
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  TRACE_START(blockIdx.x);
-  if (p.ts && tid == 0) { unsigned long long t0; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0)); atomicMin(p.ts, t0); }
-  if (tid == 0) {
-    for (int s = 0; s < stages; s++) { mbar_init(&full[s], 1); mbar_init(&empty[s], TMA_CONSUMER_WARPS); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");      // inits visible to the async proxy
-  }
-  __syncthreads();
-  if (warp == TMA_CONSUMER_WARPS) {
-    // ---- producer ----
-    if (lane == 0) {
-      int k = 0, s = 0, round = 0;
-      for (int t = blockIdx.x; t < n_tiles; t += gridDim.x, k++) {
-        if (round > 0) mbar_wait(&empty[s], (uint32_t)(round - 1) & 1u);           // every consumer warp has left this stage
-        mbar_expect_tx(&full[s], TMA_TILE_BYTES);
-        tma_load_2d(tma_smem + s * TMA_TILE_BYTES, p.tmap, (t % tiles_x) * TMA_TW, (t / tiles_x) * TMA_TH, &full[s]);
-        if (++s == stages) { s = 0; round++; }
-      }
-    }
-  } else {
-    // ---- consumers: warp w owns rows 2w, 2w+1 of every tile ----
-    const int src_pairs = p.src_h >> 1, pad_pairs = (p.coded_h - p.src_h) >> 1;
-    int s = 0, round = 0;
-    for (int t = blockIdx.x; t < n_tiles; t += gridDim.x) {
-      mbar_wait(&full[s], (uint32_t)round & 1u);
-#ifdef CSC_TRACE
-      if (t == blockIdx.x) TRACE_DATA(blockIdx.x);
-#endif
-      const uint8_t* rows = tma_smem + s * TMA_TILE_BYTES + (2 * warp) * (TMA_TW * 4);
-      const int x0 = (t % tiles_x) * TMA_TW, pr = (t / tiles_x) * (TMA_TH / 2) + warp;
-      uint4 a[2], b[2];
-#pragma unroll
-      for (int u = 0; u < 2; u++) {
-        a[u] = lds128(rows + (lane + 32 * u) * 16);
-        b[u] = lds128(rows + TMA_TW * 4 + (lane + 32 * u) * 16);
-      }
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&empty[s]);              // the stage's bytes are in registers: hand it back before computing
-      if (pr < src_pairs) {
-#pragma unroll
-        for (int u = 0; u < 2; u++) {
-          const int x = x0 + (lane + 32 * u) * 4;
-          if (x < p.coded_w) {
-            unsigned y0, y1, uv;
-            convert_quad(a[u], b[u], y0, y1, uv);
-            st_y_uv(p, x, pr, y0, y1, uv);
-            if (pr == src_pairs - 1 && pad_pairs > 0) {    // coded-size padding below the picture replicates the last row
-              convert_quad(b[u], b[u], y0, y1, uv);
-              for (int e = 1; e <= pad_pairs; e++) st_y_uv(p, x, pr + e, y0, y1, uv);
-            }
-          }
-        }
-      }
-      if (++s == stages) { s = 0; round++; }
-    }
-  }
-  if (p.ts) {
-    __syncthreads();
-    if (tid == 0) { unsigned long long t1; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1)); atomicMax(p.ts + 1, t1); }
-  }
-  TRACE_END(blockIdx.x);
 }
 
 // ---- general path: bilinear scale and/or ragged width, one thread per 2x2 output block -----
@@ -397,106 +263,24 @@ void make_taps_host(Tap* t, int dn, int sn) {
   }
 }
 
-static int g_csc_u = 2, g_csc_block = 160, g_csc_rows_per_block = 0, g_csc_tma = 0, g_csc_tma_ctas_per_sm = 2, g_csc_tma_stages = 4, g_csc_evict_first = 0, g_csc_scaled_tiled = 1;
-static void csc_env_once() {      // experiment switch, read once: B2V_CSC = ldg | ldg_ef | tma
-  static bool done = false;
-  if (done) return;
-  done = true;
-  const char* e = getenv("B2V_CSC");
-  if (!e) return;
-  if (!strcmp(e, "ldg")) { g_csc_tma = 0; g_csc_evict_first = 0; }
-  else if (!strcmp(e, "ldg_ef")) { g_csc_tma = 0; g_csc_evict_first = 1; }
-  else if (!strcmp(e, "tma")) { g_csc_tma = 1; }
-  else if (!strcmp(e, "scaled_general")) { g_csc_scaled_tiled = 0; }
-}
-extern "C" void b2v_tune_csc(int u, int block, int gy) {   // bench/tuning hook (not part of the drop-in ABI)
-  if (u > 0) g_csc_u = u;
-  if (block > 0) g_csc_block = block;
-  g_csc_rows_per_block = gy >= 0 ? gy : 0;
-  if (gy == -1) { g_csc_tma = 0; g_csc_evict_first = u >= 100; if (u >= 100) g_csc_u = u - 100; }                              // -1: LDG path, -(1 + c + 16 s): TMA path with c CTAs per SM and s stages (s = 0: unchanged)
-  if (gy <= -2) { g_csc_tma = 1; g_csc_tma_ctas_per_sm = (-gy - 1) % 16; if (-gy - 1 >= 16) g_csc_tma_stages = (-gy - 1) / 16; }
-}
-
-// ---- tensor maps: one 2-D descriptor per source buffer, built through the driver entry point (no -lcuda) and kept in DEVICE
-// memory (the TMA unit fetches it through L2; a kernel-parameter copy would be re-fetched from a new address every launch) ----
-namespace {
-using EncodeTiledFn = CUresult (*)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                                   const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-std::mutex g_map_mu;
-EncodeTiledFn g_encode = nullptr;
-bool g_encode_tried = false;
-}  // namespace
-
-void* csc_make_tensor_map(const uint8_t* d_bgra, int w, int h, int stride) {
-  {
-    std::lock_guard<std::mutex> lk(g_map_mu);
-    if (!g_encode_tried) {
-      g_encode_tried = true;
-      void* fn = nullptr; cudaDriverEntryPointQueryResult qr;
-      if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qr) == cudaSuccess && qr == cudaDriverEntryPointSuccess) g_encode = (EncodeTiledFn)fn;
-    }
-  }
-  if (!g_encode || (stride % 16) != 0 || ((uintptr_t)d_bgra % 16) != 0 || (w % 4) != 0 || (h % 2) != 0) return nullptr;
-  alignas(64) CUtensorMap m;
-  const cuuint64_t dims[2] = {(cuuint64_t)w, (cuuint64_t)h};          // elements = BGRA pixels (u32)
-  const cuuint64_t strides[1] = {(cuuint64_t)stride};
-  const cuuint32_t box[2] = {TMA_TW, TMA_TH}, estr[2] = {1, 1};
-  if (g_encode(&m, CU_TENSOR_MAP_DATA_TYPE_UINT32, 2, const_cast<uint8_t*>(d_bgra), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) return nullptr;
-  void* d = nullptr;
-  if (cudaMalloc(&d, sizeof m) != cudaSuccess) return nullptr;
-  if (cudaMemcpy(d, &m, sizeof m, cudaMemcpyHostToDevice) != cudaSuccess) { cudaFree(d); return nullptr; }
-  return d;
-}
-void csc_free_tensor_map(void* d) { if (d) cudaFree(d); }
-
-int launch_csc(const CscParams& p, int sm_count, cudaStream_t st) {
-  csc_env_once();
+int launch_csc(const CscParams& p, cudaStream_t st) {
   const bool fast = p.tx == nullptr && p.ty == nullptr && p.dst_w == p.src_w && p.dst_h == p.src_h && p.coded_w == p.dst_w &&
                     (p.coded_w % 4) == 0 && (p.src_stride % 16) == 0 && ((uintptr_t)p.src % 16) == 0 &&
                     ((uintptr_t)p.out_y % 4) == 0 && ((uintptr_t)p.out_uv % 4) == 0;
-  if (fast && p.matrix == 0 && g_csc_tma && p.tmap && (p.src_h % 2) == 0 && p.coded_h >= p.src_h) {
-    const int stages = g_csc_tma_stages, smem = stages * TMA_TILE_BYTES;
-    static int attr_smem = 0;
-    if (smem > attr_smem) { cudaFuncSetAttribute(csc_bgra_nv12_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); attr_smem = smem; }
-    const int tiles_x = (p.src_w + TMA_TW - 1) / TMA_TW, tiles_y = (p.src_h + TMA_TH - 1) / TMA_TH, n_tiles = tiles_x * tiles_y;
-    int grid = sm_count * g_csc_tma_ctas_per_sm;
-    if (grid > n_tiles) grid = n_tiles;
-    csc_bgra_nv12_tma<<<grid, TMA_THREADS, smem, st>>>(p, tiles_x, n_tiles, stages);
-    return 1;
-  }
   if (fast) {
     int quads = p.coded_w / 4, pairs = p.coded_h / 2;
-    int block = g_csc_block;
-    while (block > 32 && quads % block != 0 && block > 64) block -= 32;   // prefer a divisor of the row
-    if (quads % block != 0) block = g_csc_block;
+    int block = CSC_BLOCK;
+    while (quads % block != 0 && block > 64) block -= 32;   // prefer a divisor of the row
+    if (quads % block != 0) block = CSC_BLOCK;
     int gx = (quads + block - 1) / block;
-    int U = g_csc_u;
-    int groups = (pairs + U - 1) / U;
-    int gy = g_csc_rows_per_block > 0 ? g_csc_rows_per_block : groups;   // default: one U-group per block
-    if (gy > groups) gy = groups;
+    int gy = (pairs + CSC_U - 1) / CSC_U;                    // one U-group per block
     if (gy > 65535) gy = 65535;
     dim3 grid(gx, gy);
-    if (p.matrix == 1) {
-      csc_bgra_nv12_fast<2, false, 1><<<grid.y == (unsigned)gy && U == 2 ? grid : dim3(gx, (pairs + 1) / 2), block, 0, st>>>(p, quads, pairs);
-    } else if (g_csc_evict_first) {
-      switch (U) {
-        case 1: csc_bgra_nv12_fast<1, true><<<grid, block, 0, st>>>(p, quads, pairs); break;
-        case 2: csc_bgra_nv12_fast<2, true><<<grid, block, 0, st>>>(p, quads, pairs); break;
-        case 3: csc_bgra_nv12_fast<3, true><<<grid, block, 0, st>>>(p, quads, pairs); break;
-        default: csc_bgra_nv12_fast<4, true><<<grid, block, 0, st>>>(p, quads, pairs); break;
-      }
-    } else {
-      switch (U) {
-        case 1: csc_bgra_nv12_fast<1, false><<<grid, block, 0, st>>>(p, quads, pairs); break;
-        case 2: csc_bgra_nv12_fast<2, false><<<grid, block, 0, st>>>(p, quads, pairs); break;
-        case 3: csc_bgra_nv12_fast<3, false><<<grid, block, 0, st>>>(p, quads, pairs); break;
-        default: csc_bgra_nv12_fast<4, false><<<grid, block, 0, st>>>(p, quads, pairs); break;
-      }
-    }
+    if (p.matrix == 1) csc_bgra_nv12_fast<1><<<grid, block, 0, st>>>(p, quads, pairs);
+    else csc_bgra_nv12_fast<0><<<grid, block, 0, st>>>(p, quads, pairs);
   } else {
     // scaled: the tiled kernel when the tile's source footprint fits shared memory (any sane scale factor), else the general one
-    if (p.tx && p.ty && g_csc_scaled_tiled && (p.src_stride % 16) == 0 && ((uintptr_t)p.src % 16) == 0) {
+    if (p.tx && p.ty && (p.src_stride % 16) == 0 && ((uintptr_t)p.src % 16) == 0) {
       const long long fw = ((long long)SC_TW * p.src_w + p.dst_w - 1) / p.dst_w + 8, fh = ((long long)SC_TH * p.src_h + p.dst_h - 1) / p.dst_h + 3;
       const int fw_cap = (int)((fw + 3) & ~3LL), fh_cap = (int)fh;
       const long long smem = (long long)fw_cap * fh_cap * 4;

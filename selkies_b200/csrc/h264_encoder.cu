@@ -1,6 +1,6 @@
 // h264_encoder.cu — host side of the H.264 Constrained-Baseline encoder: parameter sets (7.3.2.1/2),
 // HBM buffers, per-picture sequencing (frame_num, idr_pic_id, reference swap) and the kernel pipeline
-//   [k_intra_rows | k_inter_mb] -> k_cavlc_mb -> k_slice_scan -> k_slice_copy -> k_slice_ep -> k_pack_au
+//   [k_intra_rows | k_inter_mb] -> k_cavlc_mb -> k_slice_build -> k_pack_au
 // The output format is what the reference's consumers require (SURVEY.md §8 a13): Annex-B, CAVLC,
 // no B-frames, 4:2:0, in-band SPS/PPS on every IDR (src/selkies/rtc.py:394-401,
 // src/selkies/webrtc/codecs/h264.py:281-321).
@@ -291,8 +291,7 @@ int encoder_encode(Encoder* e, const EncodeFrameParams* p, cudaStream_t st) {
   }
   n += launch_cavlc(f, sp);
   if (p->ev) cudaEventRecord(p->ev[3], st);
-  n += launch_slice_scan(f, sp);
-  n += launch_slice_copy_ep(f, sp);
+  n += launch_slice_build(f, sp);
   if (p->ev) cudaEventRecord(p->ev[4], st);
   n += launch_pack_cap(f, (long long)e->au_cap, sp);
   if (p->ev) cudaEventRecord(p->ev[5], st);

@@ -13,14 +13,11 @@
 //   k_pack_au     one block per slice: prefix over slice sizes, emulation prevention (parallel rule: a 03 is
 //                 inserted before byte i iff byte<=3 and the run of zero bytes before it is even and >=2),
 //                 start codes + NAL headers, AuHeader, band table.
-// (k_slice_build_v1 — one block per slice, the three phases in sequence — is kept for A/B runs: B2V_SLICE_KERNEL=v1.)
 // CPU restatement: oracle/h264_ref.c cavlc_block(), code_slice(), nal_write(), rc_update().
 #include "h264_common.cuh"
 #include "h264_cavlc.cuh"
 #include "h264_encoder.h"
 #include "h264_kernels.h"
-#include <cstdlib>
-#include <cstring>
 
 namespace b2v {
 
@@ -290,164 +287,7 @@ __device__ __forceinline__ void rc_step(const FrameCtx& f, int qp_used, long lon
   rc->fb[f.pic & 1] = n;
 }
 
-// ---- k_slice_scan: one block per slice.  Block-wide scans give every macroblock (a) its mb_skip_run and (b) the bit
-// offset of its first bit inside the slice RBSP.  Nothing is copied here, so a slice of many macroblock rows costs one
-// short loop iteration per 256 macroblocks.
-__device__ __forceinline__ void slice_scan_body(const FrameCtx& f) {
-  __shared__ long long s_warp_sum[SLICE_THREADS / 32];
-  __shared__ int s_warp_max[SLICE_THREADS / 32];
-  __shared__ long long s_carry_bits;
-  __shared__ bool s_is_last;
-  __shared__ int s_carry_last;      // index (within the slice) of the last non-skipped macroblock seen so far
-  __shared__ uint32_t s_nb[SLICE_THREADS];
-  __shared__ int s_run[SLICE_THREADS];
-  __shared__ long long s_off[SLICE_THREADS];
-  const int s = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const SliceGeo geo = slice_geo(f, s);
-  const int row0 = geo.row0, mb0 = geo.mb0, n_mb = geo.n_mb;
-  const int qp = frame_qp(f);
-  uint32_t* out = f.slice_buf + (size_t)s * f.slice_words;
-  if (tid == 0) {
-    GlobalSink g{out, 0};
-    const int band = row0 / f.band_rows;      // first_mb_in_slice and frame_num are the band's own
-    slice_header(g, f, mb0 - band * f.band_rows * f.mbw, qp, f.idr ? 0 : f.striped ? f.band_fn[band] : f.frame_num);
-    s_carry_bits = g.pos; s_carry_last = -1;
-  }
-  __syncthreads();
-  for (int base = 0; base < n_mb; base += SLICE_THREADS) {
-    const int i = base + tid;
-    uint32_t nbits = 0; bool skip = true, pcm = false;
-    if (i < n_mb) { const uint32_t v = f.mb_nbits[mb0 + i]; skip = (v >> 31) != 0; pcm = ((v >> 30) & 1u) != 0; nbits = v & 0x3fffffffu; }
-    // I_PCM samples must start byte-aligned in the RBSP, so a macroblock's length then depends on its position:
-    // chunks containing one (pathological content only) get their offsets from a serial walk below.
-    const bool any_pcm = __syncthreads_or(pcm) != 0;
-    int incl_max = skip ? -1 : i;     // last non-skipped index up to and including i (max-scan)
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) { const int o = __shfl_up_sync(FULL, incl_max, d); if (lane >= d) incl_max = max(incl_max, o); }
-    if (lane == 31) s_warp_max[warp] = incl_max;
-    __syncthreads();
-    int prev_max = s_carry_last;
-    for (int w = 0; w < warp; w++) prev_max = max(prev_max, s_warp_max[w]);
-    int excl_max = __shfl_up_sync(FULL, incl_max, 1);
-    if (lane == 0) excl_max = -1;
-    excl_max = max(excl_max, prev_max);
-    const int run = i - 1 - excl_max;                      // mb_skip_run in front of macroblock i
-    const int pre = (!skip && !f.idr) ? ue_len((uint32_t)run) : 0;
-    const long long tot = skip ? 0 : (long long)pre + nbits;
-    long long incl = tot;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) { const long long o = __shfl_up_sync(FULL, incl, d); if (lane >= d) incl += o; }
-    if (lane == 31) s_warp_sum[warp] = incl;
-    __syncthreads();
-    const long long chunk_base = s_carry_bits;
-    long long woff = chunk_base;
-    for (int w = 0; w < warp; w++) woff += s_warp_sum[w];
-    long long my_off = woff + incl - tot;
-    if (any_pcm) { s_nb[tid] = skip ? 0xffffffffu : (nbits | (pcm ? 0x40000000u : 0u)); s_run[tid] = run; }
-    __syncthreads();
-    if (tid == SLICE_THREADS - 1) {
-      long long t = chunk_base;
-      for (int w = 0; w < SLICE_THREADS / 32; w++) t += s_warp_sum[w];
-      if (!any_pcm) s_carry_bits = t;
-      int m = s_carry_last;
-      for (int w = 0; w < SLICE_THREADS / 32; w++) m = max(m, s_warp_max[w]);
-      s_carry_last = m;
-    }
-    if (any_pcm) {
-      if (tid == 0) {
-        long long pos = chunk_base;
-        for (int j = 0; j < SLICE_THREADS && base + j < n_mb; j++) {
-          const uint32_t nb = s_nb[j];
-          if (nb == 0xffffffffu) continue;
-          s_off[j] = pos;
-          pos += (f.idr ? 0 : ue_len((uint32_t)s_run[j])) + (nb & 0x3fffffffu);
-          if (nb & 0x40000000u) pos = ((pos + 7) & ~7LL) + 384 * 8;
-        }
-        s_carry_bits = pos;
-      }
-      __syncthreads();
-      my_off = s_off[tid];
-    }
-    if (i < n_mb) { f.mb_off[mb0 + i] = my_off; f.mb_run[mb0 + i] = run; }
-    __syncthreads();
-  }
-  // trailing mb_skip_run, rbsp_trailing_bits
-  if (tid == 0) {
-    GlobalSink g{out, s_carry_bits};
-    if (!f.idr) { const int run = n_mb - 1 - s_carry_last; if (run > 0) put_ue(g, (uint32_t)run); }
-    f.slice_bits[s] = g.pos;
-    if (s_carry_last >= 0) {                          // benign races: every writer stores the same value
-      f.rc->pic_coded = 1;
-      if (f.striped) f.band_coded[row0 / f.band_rows] = 1;
-    }
-    g.put(1, 1);
-    f.slice_rbsp[s] = (uint32_t)((g.pos + 7) >> 3);
-    // last block of the picture to get here runs the rate-control step (every block read its QP from the controller at its
-    // start, i.e. before this point, so the update cannot disturb a block still running)
-    __threadfence();
-    s_is_last = atomicAdd(&f.rc->scan_done, 1) == f.n_slices - 1;
-  }
-  __syncthreads();
-  if (s_is_last) {
-    __threadfence();
-    long long bits = 0;
-    for (int j = tid; j < f.n_slices; j += SLICE_THREADS) bits += __ldcg(&f.slice_bits[j]);
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) bits += __shfl_xor_sync(FULL, bits, d);
-    if (lane == 0) s_warp_sum[warp] = bits;
-    __syncthreads();
-    if (tid == 0) {
-      long long t = 0;
-      for (int w = 0; w < SLICE_THREADS / 32; w++) t += s_warp_sum[w];
-      f.rc->scan_done = 0;
-      rc_step(f, qp, t);
-    }
-  }
-}
-
-// ---- k_slice_copy: COPY_LANES threads per macroblock shift its bit string (mb_skip_run prefix, CAVLC words, or the
-// 384 raw samples of an I_PCM macroblock) into the slice RBSP with atomicOr.  Fully parallel over the picture.
-constexpr int COPY_LANES = 8;
-constexpr int COPY_THREADS = 256;
-
-__device__ __forceinline__ void slice_copy_body(const FrameCtx& f) {
-  const int s = blockIdx.x, sub = threadIdx.x % COPY_LANES;
-  const SliceGeo geo = slice_geo(f, s);
-  uint32_t* out = f.slice_buf + (size_t)s * f.slice_words;
-  for (int i = threadIdx.x / COPY_LANES; i < geo.n_mb; i += COPY_THREADS / COPY_LANES) {
-  const int mb = geo.mb0 + i;                                // the macroblocks of a slice are consecutive (whole rows, or a piece of one row)
-  const uint32_t v = f.mb_nbits[mb];
-  if (v >> 31) continue;                                     // P_Skip: folded into a later mb_skip_run
-  const bool pcm = ((v >> 30) & 1u) != 0;
-  const uint32_t nbits = v & 0x3fffffffu;
-  const int mby = mb / f.mbw, mbx = mb - mby * f.mbw;
-  long long pos = f.mb_off[mb];
-  if (!f.idr) {
-    const uint32_t run = (uint32_t)f.mb_run[mb];
-    if (sub == 0) { GlobalSink g{out, pos}; put_ue(g, run); }
-    pos += ue_len(run);
-  }
-  const uint32_t* src = f.mb_words + (size_t)mb * MB_WORDS;
-  for (int w = sub; w < (int)((nbits + 31) >> 5); w += COPY_LANES) or_word(out, pos + 32LL * w, src[w]);
-  if (pcm) {     // I_PCM payload: 256 luma, 64 Cb, 64 Cr samples from the reconstruction (== source), byte aligned
-    const long long pp = (pos + nbits + 7) & ~7LL;
-    const int px = mbx * 16, py = mby * 16;
-    const uint8_t* ry = f.recon; const uint8_t* ruv = f.recon + (size_t)f.cw * f.ch;
-    for (int w = sub; w < 96; w += COPY_LANES) {
-      uint32_t q;
-      if (w < 64) q = __byte_perm(__ldcg(reinterpret_cast<const uint32_t*>(ry + (size_t)(py + (w >> 2)) * f.cw + px + (w & 3) * 4)), 0, 0x0123);
-      else {
-        const int k = (w - 64) & 15, comp = (w - 64) >> 4;
-        const uint2 c2 = __ldcg(reinterpret_cast<const uint2*>(ruv + (size_t)(py / 2 + (k >> 1)) * f.cw + px + (k & 1) * 8));
-        q = comp == 0 ? __byte_perm(c2.x, c2.y, 0x0246) : __byte_perm(c2.x, c2.y, 0x1357);
-      }
-      or_word(out, pp + 32LL * w, q);
-    }
-  }
-  }
-}
-
-// ---- k_slice_ep: one block per slice counts the emulation-prevention bytes the slice needs (7.4.1): a 03 goes in
+// ---- slice_ep_body: one block counts the emulation-prevention bytes slice s needs (7.4.1): a 03 goes in
 // front of byte i iff byte <= 3 and the run of zero bytes before it is even and >= 2.
 __device__ __forceinline__ void slice_ep_body(const FrameCtx& f, int s) {
   __shared__ int s_red[SLICE_THREADS / 32];
@@ -480,22 +320,7 @@ __device__ __forceinline__ void slice_ep_body(const FrameCtx& f, int s) {
   }
 }
 
-// ---- k_slice_build: the three per-slice stages in ONE launch (they only ever depended on each other inside a slice): scan ->
-// copy -> emulation-prevention count.  The block's own global writes (macroblock offsets, the RBSP words built with atomicOr) are
-// visible to it after a fence + barrier.
-static_assert(SLICE_THREADS == COPY_THREADS, "one block shape for the fused slice kernel");
-__global__ void __launch_bounds__(SLICE_THREADS) k_slice_build_v1(FrameCtx f) {
-  slice_scan_body(f);
-  __threadfence();
-  __syncthreads();
-  slice_copy_body(f);
-  __threadfence();
-  __syncthreads();
-  slice_ep_body(f, blockIdx.x);
-}
-
-
-// ---- k_slice_build (chunked): one block per CHUNK of up to 256 consecutive macroblocks of a slice, so a slice of many rows is built
+// ---- k_slice_build: one block per CHUNK of up to 256 consecutive macroblocks of a slice, so a slice of many rows is built
 // by many blocks instead of one long loop.  What a chunk needs from the chunks in front of it is (a) the bit position where it starts
 // and (b) the mb_skip_run still open at that point — the first coded macroblock of a chunk codes ue(open run + its own leading skips),
 // whose LENGTH is the only thing in a chunk that depends on the carry.  Decoupled look-back (the chunks of a slice are consecutive
@@ -509,6 +334,7 @@ __global__ void __launch_bounds__(SLICE_THREADS) k_slice_build_v1(FrameCtx f) {
 struct ChunkAgg { int flag; int has; int first_run; int trailing; long long rest_bits; };   // has: bit 0 coded macroblock present, bit 1 I_PCM inside (no aggregate)
 struct ChunkInc { int flag; int trailing; long long bits; };
 constexpr int CHUNK_MAX_POLLS = 1 << 22;
+constexpr int COPY_LANES = 8;      // threads per macroblock in the bit-string copy
 
 __device__ __forceinline__ bool wait_flag(const volatile int* flag, int tag) {
   int spins = 0;
@@ -749,7 +575,7 @@ __global__ void __launch_bounds__(PACK_THREADS) k_pack_au(FrameCtx f, long long 
   __shared__ int s_wsum[PACK_THREADS / 32];
   __shared__ int s_carry;
   const int s = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  // the controller has already moved on to the next picture (rc_step ran in k_slice_scan, before this kernel and possibly on another
+  // the controller has already moved on to the next picture (rc_step ran in k_slice_build, before this kernel and possibly on another
   // stream): this picture's QP is the one it recorded
   const int qp = f.rc->last_qp;
   // byte offset of this slice's NAL inside the access unit
@@ -865,18 +691,12 @@ int launch_cavlc(const FrameCtx& f, cudaStream_t st) {
   k_cavlc_mb<<<(mbs + CAVLC_WARPS - 1) / CAVLC_WARPS, 32 * CAVLC_WARPS, 0, st>>>(f);
   return 1;
 }
-int launch_slice_scan(const FrameCtx& f, cudaStream_t st) {
-  static const bool v1 = getenv("B2V_SLICE_KERNEL") && !strcmp(getenv("B2V_SLICE_KERNEL"), "v1");   // A/B: one block per slice
-  if (v1) { k_slice_build_v1<<<f.n_slices, SLICE_THREADS, 0, st>>>(f); return 1; }
+int launch_slice_build(const FrameCtx& f, cudaStream_t st) {
   FrameCtx g = f;
   const int full = f.seg_cols ? f.seg_cols : f.slice_rows * f.mbw;       // macroblocks of a full-size slice of this picture
   g.chunks_per_slice = (full + SLICE_THREADS - 1) / SLICE_THREADS;
   k_slice_build<<<f.n_slices * g.chunks_per_slice, SLICE_THREADS, 0, st>>>(g);      // scan + copy + emulation-prevention count
   return 1;
-}
-int launch_slice_copy_ep(const FrameCtx& f, cudaStream_t st) {
-  (void)f; (void)st;          // folded into k_slice_build (launch_slice_scan)
-  return 0;
 }
 int launch_pack_cap(const FrameCtx& f, long long au_cap, cudaStream_t st) {
   k_pack_au<<<f.n_slices, PACK_THREADS, 0, st>>>(f, au_cap);

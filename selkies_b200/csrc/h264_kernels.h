@@ -6,7 +6,6 @@ struct FrameCtx;
 int launch_intra(const FrameCtx& f, cudaStream_t st);    // IDR: Intra16x16 rows (h264_intra.cu)
 int launch_inter(const FrameCtx& f, cudaStream_t st);    // P: motion search + residual (h264_inter.cu)
 int launch_cavlc(const FrameCtx& f, cudaStream_t st);    // per-macroblock CAVLC bit strings (h264_entropy.cu)
-int launch_slice_scan(const FrameCtx& f, cudaStream_t st);      // k_slice_scan; its last block runs the rate-control step (h264_entropy.cu)
-int launch_slice_copy_ep(const FrameCtx& f, cudaStream_t st);   // k_slice_copy + k_slice_ep
+int launch_slice_build(const FrameCtx& f, cudaStream_t st);     // slice RBSP + emulation-prevention count; its last block runs the rate-control step
 int launch_pack_cap(const FrameCtx& f, long long au_cap, cudaStream_t st);   // emulation prevention + AU assembly
 }  // namespace b2v

@@ -1,5 +1,5 @@
 """A dozen 4K CSC launches over distinct resident frames (CSC-only session) — the target of bench.py's live ncu traffic probe
-and of the `ncu --set full` captures under profiles/.  CSC_KERNEL=ldg|tma1|tma2 selects the kernel (default: the library's)."""
+and of the `ncu --set full` captures under profiles/.  CSC_SIZE=8k runs 7680x4320 instead."""
 import os
 import sys
 
@@ -10,9 +10,6 @@ from selkies_b200.session import Session        # noqa: E402
 from tests import synth                         # noqa: E402
 
 W, H = (7680, 4320) if os.environ.get("CSC_SIZE") == "8k" else (3840, 2160)
-k = os.environ.get("CSC_KERNEL")
-if k:
-    N.lib().b2v_tune_csc(2, 160, {"ldg": -1, "tma1": -2, "tma2": -3}[k])
 with Session(W, H, flags=N.B2V_FLAG_NO_ENCODE) as s:
     for i in range(4):
         s.resident_upload(i, synth.desktop(W, H, i))

@@ -1,6 +1,6 @@
 """In-step numbers for the 4K headline workload with the library built as it is: pictures/s (inputs resident, no timing flags),
 the CSC launch by CUDA-event pair and by the kernel's own %globaltimer stamps, and the per-stage event breakdown.
-Run on the GPU box: [B2V_CSC=ldg|ldg_ef|tma] python tools/instep.py [n_pictures]"""
+Run on the GPU box: python tools/instep.py [n_pictures]"""
 import json
 import os
 import sys
@@ -15,7 +15,7 @@ W, H, ND = 3840, 2160, 16
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 512
 CONTENT = os.environ.get("B2V_CONTENT", "desktop")      # desktop (headline) | gradient (S4) | noise (S2)
 frames = [{"desktop": synth.desktop, "gradient": synth.gradient}[CONTENT](W, H, t) if CONTENT != "noise" else synth.noise(W, H, 100 + t) for t in range(ND)]
-out = {"env": os.environ.get("B2V_CSC", "default")}
+out = {}
 
 
 def run(flags, label):
