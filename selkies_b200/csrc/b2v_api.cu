@@ -46,6 +46,7 @@ namespace {
 constexpr int kMaxSlots = 16;
 constexpr int kOutHead = 64;              // bytes reserved in front of the AU in the pinned output slot
 constexpr size_t kFirstChunk = 256 << 10; // AU bytes fetched speculatively with the size word
+constexpr int kTimingEvents = 6;          // around the CSC, then after each H.264 stage (EncodeFrameParams::ev)
 
 struct Job {
   int out_idx; int in_slot; int frame_id; int is_key; int64_t capture_ns; int64_t pts; int hdr_w, hdr_h;
@@ -86,7 +87,7 @@ enum : uint8_t { SLOT_FREE = 0, SLOT_ACQUIRED = 1, SLOT_IN_FLIGHT = 2 };
 
 struct Session {
   b2v_settings cfg{};
-  int device = 0, sm_count = 148;
+  int device = 0;
   int src_w = 0, src_h = 0, dst_w = 0, dst_h = 0, coded_w = 0, coded_h = 0;
   bool encode = true, timing = false, timing_csc_only = false;
   cudaStream_t st_copy = nullptr, st_enc = nullptr, st_out = nullptr, st_pack = nullptr;
@@ -114,7 +115,8 @@ struct Session {
   cudaEvent_t ev_enc[kMaxSlots] = {}, ev_out[kMaxSlots] = {};
   bool out_free[kMaxSlots] = {};
   size_t au_cap = 0;
-  int au_data_off = 64, n_bands = 0;   // bytes in front of the first NAL in d_au (AuHeader [+ band table]); bands when striped
+  int au_data_off = 64, n_bands = 0;   // bytes in front of the first NAL in d_au (AuHeader [+ band table]); bands in that table
+  int band_h = 0;                      // pixel rows per band (the coded height when full-frame: one band, no table)
   int out_next = 0;
   int ring_next = 0;
   cudaEvent_t ev_timer[2] = {};
@@ -128,8 +130,8 @@ struct Session {
   int bitrate_kbps = 8000;
   int qp_fixed = 26;
 
-  // timing events (B2V_FLAG_TIMING): 8 per output slot, read back by the output thread
-  cudaEvent_t ev_t[kMaxSlots][8] = {};
+  // timing events (B2V_FLAG_TIMING): per output slot, read back by the output thread
+  cudaEvent_t ev_t[kMaxSlots][kTimingEvents] = {};
 
   b2v_cb cb = nullptr; void* user = nullptr;
   std::mutex mu;                 // guards everything below + sequencing state
@@ -145,6 +147,9 @@ struct Session {
 };
 
 int round16(int v) { return (v + 15) & ~15; }
+
+// source and encoded sizes a session accepts: even, 16..7680 x 16..4320 (the reference's maximum, selkies.py:281)
+bool size_supported(int w, int h) { return w >= 16 && h >= 16 && w <= 7680 && h <= 4320 && !(w & 1) && !(h & 1); }
 
 int alloc_geometry(Session* s) {
   // (re)allocate everything that depends on the frame size
@@ -177,15 +182,11 @@ int alloc_geometry(Session* s) {
     s->au_cap = jpeg_au_capacity(s->jenc);
     s->au_data_off = jpeg_au_data_offset(s->jenc);
     s->n_bands = jpeg_stripe_count(s->jenc);
-    for (int i = 0; i < s->n_slots; i++) {
-      CK(cudaMalloc((void**)&s->d_au[i], s->au_cap));
-      CK(cudaHostAlloc((void**)&s->h_out[i], s->au_cap + kOutHead, cudaHostAllocDefault));
-    }
+    s->band_h = jpeg_stripe_rows(s->jenc) * 16;
   } else if (s->encode) {
     EncoderConfig ec{};
     ec.width = s->dst_w; ec.height = s->dst_h; ec.coded_w = s->coded_w; ec.coded_h = s->coded_h;
     ec.slice_rows = s->cfg.slice_rows;          // <= 0: the encoder's default rule
-    ec.sm_count = s->sm_count;
     ec.stripe_rows = s->cfg.stripe_rows > 0 ? s->cfg.stripe_rows : 0;
     ec.idr_slice_mbs = s->cfg.idr_slice_mbs;
     int rc = encoder_create(&ec, &s->enc);
@@ -193,6 +194,9 @@ int alloc_geometry(Session* s) {
     s->au_cap = encoder_au_capacity(s->enc);
     s->au_data_off = encoder_au_data_offset(s->enc);
     s->n_bands = encoder_band_count(s->enc);
+    s->band_h = s->n_bands > 0 ? s->cfg.stripe_rows * 16 : s->coded_h;
+  }
+  if (s->encode) {
     for (int i = 0; i < s->n_slots; i++) {
       CK(cudaMalloc((void**)&s->d_au[i], s->au_cap));
       CK(cudaHostAlloc((void**)&s->h_out[i], s->au_cap + kOutHead, cudaHostAllocDefault));
@@ -230,6 +234,16 @@ CscParams csc_params(Session* s, const uint8_t* d_bgra, int stride, uint8_t* d_n
   return p;
 }
 
+// 10-byte pixelflux stripe header in front of an H.264 band: 0x04 | is_key | frame_id | y_start | width | height, u16be each
+uint8_t* put_stripe_header(uint8_t* h, const Job& j, int y0, int bh) {
+  h[0] = 0x04; h[1] = j.is_key ? 1 : 0;
+  h[2] = (uint8_t)(j.frame_id >> 8); h[3] = (uint8_t)j.frame_id;
+  h[4] = (uint8_t)(y0 >> 8); h[5] = (uint8_t)y0;
+  h[6] = (uint8_t)(j.hdr_w >> 8); h[7] = (uint8_t)j.hdr_w;
+  h[8] = (uint8_t)(bh >> 8); h[9] = (uint8_t)bh;
+  return h;
+}
+
 void output_loop(Session* s) {
   cudaSetDevice(s->device);
   prctl(PR_SET_TIMERSLACK, 1000UL, 0, 0, 0);     // this thread's short sleeps (wait_event_polling) are not rounded up by 50 us
@@ -246,7 +260,6 @@ void output_loop(Session* s) {
       j = s->jobs.front(); s->jobs.pop_front();
     }
     int size = 0, qp = 0;
-    const uint8_t* data = nullptr;
     int64_t ns_event = 0, ns_cb = 0; bool slept = false;
     if (s->encode) {
       const int64_t tw = now_ns();
@@ -271,18 +284,6 @@ void output_loop(Session* s) {
         cudaStreamSynchronize(s->st_out);
         std::lock_guard<std::mutex> lk(s->mu);
         s->stats.d2h_bytes += (int64_t)(doff + size - have);
-      }
-      uint8_t* au = base + doff;
-      data = au;
-      if (s->n_bands == 0 && s->cfg.header_mode == B2V_HDR_PIXELFLUX) {
-        // 10-byte stripe header written into the slack in front of the AU (AuHeader is 64 bytes; already consumed)
-        uint8_t* h = au - 10;
-        h[0] = 0x04; h[1] = j.is_key ? 1 : 0;
-        h[2] = (uint8_t)(j.frame_id >> 8); h[3] = (uint8_t)j.frame_id;
-        h[4] = 0; h[5] = 0;
-        h[6] = (uint8_t)(j.hdr_w >> 8); h[7] = (uint8_t)j.hdr_w;
-        h[8] = (uint8_t)(j.hdr_h >> 8); h[9] = (uint8_t)j.hdr_h;
-        data = h; size += 10;
       }
     } else {
       const int64_t tw = now_ns();
@@ -313,15 +314,17 @@ void output_loop(Session* s) {
       }
       s->stats.ms_total_gpu += ms[5];
     }
-    if (s->encode && size > 0 && s->n_bands > 0) {
-      // striped mode: one callback per band that carries data, in picture order.  The band table is copied out first:
-      // the 10-byte header of band k is written over the tail of band k-1 (already delivered) or the table slack.
-      std::vector<BandEntry> tab(s->n_bands);
-      memcpy(tab.data(), s->h_out[j.out_idx] + sizeof(AuHeader), sizeof(BandEntry) * s->n_bands);
+    if (s->encode && size > 0) {
+      // one callback per band that carries data, in picture order; a full-frame picture is one band that spans the access
+      // unit, and the device writes no table for it.  The table is copied out first: the 10-byte header of band k is written
+      // over the tail of band k-1 (already delivered) or the slack in front of the first NAL (table or AuHeader, both consumed).
+      std::vector<BandEntry> tab(s->n_bands > 0 ? s->n_bands : 1);
+      if (s->n_bands > 0) memcpy(tab.data(), s->h_out[j.out_idx] + sizeof(AuHeader), sizeof(BandEntry) * s->n_bands);
+      else tab[0] = BandEntry{0, size, 1, 0};
       uint8_t* au = s->h_out[j.out_idx] + s->au_data_off;
-      const int rows = (s->jpeg ? jpeg_stripe_rows(s->jenc) : s->cfg.stripe_rows) * 16;
+      const int rows = s->band_h;
       int delivered_bytes = 0;
-      for (int b = 0; b < s->n_bands; b++) {
+      for (int b = 0; b < (int)tab.size(); b++) {
         const BandEntry& be = tab[b];
         if (!be.coded || be.size <= 0 || (long long)be.off + be.size > size) continue;
         const int y0 = b * rows, bh = (y0 + rows <= j.hdr_h) ? rows : j.hdr_h - y0;
@@ -334,13 +337,7 @@ void output_loop(Session* s) {
           h[0] = (uint8_t)(j.frame_id >> 8); h[1] = (uint8_t)j.frame_id; h[2] = (uint8_t)(y0 >> 8); h[3] = (uint8_t)y0;
           f.data = h; f.size += 4;
         } else if (s->cfg.header_mode == B2V_HDR_PIXELFLUX) {
-          uint8_t* h = au + be.off - 10;
-          h[0] = 0x04; h[1] = j.is_key ? 1 : 0;
-          h[2] = (uint8_t)(j.frame_id >> 8); h[3] = (uint8_t)j.frame_id;
-          h[4] = (uint8_t)(y0 >> 8); h[5] = (uint8_t)y0;
-          h[6] = (uint8_t)(j.hdr_w >> 8); h[7] = (uint8_t)j.hdr_w;
-          h[8] = (uint8_t)(bh >> 8); h[9] = (uint8_t)bh;
-          f.data = h; f.size += 10;
+          f.data = put_stripe_header(au + be.off - 10, j, y0, bh); f.size += 10;
         }
         f.frame_id = j.frame_id; f.is_key = j.is_key; f.qp = qp; f.pts90k = j.pts; f.capture_ns = j.capture_ns;
         f.y_start = y0; f.height = bh;
@@ -348,11 +345,6 @@ void output_loop(Session* s) {
         if (s->cb) { const int64_t tc = now_ns(); s->cb(&f, s->user); ns_cb += now_ns() - tc; }
       }
       size = delivered_bytes;
-    } else if (s->cb && s->encode && size > 0) {
-      b2v_frame f{};
-      f.data = data; f.size = size; f.frame_id = j.frame_id; f.is_key = j.is_key; f.qp = qp;
-      f.pts90k = j.pts; f.capture_ns = j.capture_ns; f.y_start = 0; f.height = j.hdr_h;
-      const int64_t tc = now_ns(); s->cb(&f, s->user); ns_cb = now_ns() - tc;
     }
     {
       std::lock_guard<std::mutex> lk(s->mu);
@@ -442,23 +434,19 @@ int submit_common(Session* s, const uint8_t* d_bgra, int stride, int in_slot, in
   int nl = launch_csc(cp, s->st_enc);
   if (ev) cudaEventRecord(ev[1], s->st_enc);
   if (in_slot >= 0) CKS(cudaEventRecord(s->ev_csc[in_slot], s->st_enc));
-  CKS(cudaEventRecord(s->ev_enc[out_idx], s->st_enc));
+  cudaStream_t st_done = s->st_enc;       // the picture's last work (the CSC in B2V_FLAG_NO_ENCODE mode) completes here
   if (s->encode && s->jpeg) {
     nl += jpeg_encode(s->jenc, s->d_cur, s->d_au[out_idx], j.is_key, s->st_enc);
-    CKS(cudaEventRecord(s->ev_enc[out_idx], s->st_enc));
-    CKS(cudaStreamWaitEvent(s->st_out, s->ev_enc[out_idx], 0));
-    size_t first = s->au_cap < kFirstChunk ? s->au_cap : kFirstChunk;
-    CKS(cudaMemcpyAsync(s->h_out[out_idx], s->d_au[out_idx], first, cudaMemcpyDeviceToHost, s->st_out));
-    CKS(cudaEventRecord(s->ev_out[out_idx], s->st_out));
-    std::lock_guard<std::mutex> lk(s->mu);
-    s->stats.d2h_bytes += (int64_t)first;
   } else if (s->encode) {
     fp.cur = s->d_cur; fp.au = s->d_au[out_idx]; fp.ev = s->timing_csc_only ? nullptr : ev; fp.csc_ts = cp.ts;
     fp.st_pack = fp.ev ? nullptr : s->st_pack;      // per-stage events need the serial schedule
     nl += encoder_encode(s->enc, &fp, s->st_enc);
-    CKS(cudaEventRecord(s->ev_enc[out_idx], fp.st_pack ? fp.st_pack : s->st_enc));      // the access unit is complete here
+    if (fp.st_pack) st_done = fp.st_pack;
+  }
+  CKS(cudaEventRecord(s->ev_enc[out_idx], st_done));
+  if (s->encode) {
     CKS(cudaStreamWaitEvent(s->st_out, s->ev_enc[out_idx], 0));
-    size_t first = s->au_cap < kFirstChunk ? s->au_cap : kFirstChunk;
+    const size_t first = s->au_cap < kFirstChunk ? s->au_cap : kFirstChunk;
     CKS(cudaMemcpyAsync(s->h_out[out_idx], s->d_au[out_idx], first, cudaMemcpyDeviceToHost, s->st_out));
     CKS(cudaEventRecord(s->ev_out[out_idx], s->st_out));
     std::lock_guard<std::mutex> lk(s->mu);
@@ -485,7 +473,7 @@ void release_session(Session* s) {
     if (s->ev_csc[i]) cudaEventDestroy(s->ev_csc[i]);
     if (s->ev_enc[i]) cudaEventDestroy(s->ev_enc[i]);
     if (s->ev_out[i]) cudaEventDestroy(s->ev_out[i]);
-    for (int k = 0; k < 8; k++) if (s->ev_t[i][k]) cudaEventDestroy(s->ev_t[i][k]);
+    for (int k = 0; k < kTimingEvents; k++) if (s->ev_t[i][k]) cudaEventDestroy(s->ev_t[i][k]);
   }
   if (s->ev_timer[0]) cudaEventDestroy(s->ev_timer[0]);
   if (s->ev_timer[1]) cudaEventDestroy(s->ev_timer[1]);
@@ -495,6 +483,40 @@ void release_session(Session* s) {
   if (s->st_out) cudaStreamDestroy(s->st_out);
   if (s->st_pack) cudaStreamDestroy(s->st_pack);
   delete s;
+}
+
+// b2v_bench_csc / b2v_bench_csc_burst: `iters` CSC launches cycling over the first n_resident resident frames.  per_launch:
+// each launch is bracketed by its own event pair and the mean excludes host launch gaps; otherwise one pair brackets the burst.
+int bench_csc(Session* s, int n_resident, int iters, bool per_launch, float* ms_per_launch) {
+  if (!s || n_resident <= 0 || n_resident > (int)s->resident.size() || iters <= 0 || !ms_per_launch) return fail(B2V_EINVAL, "bad argument");
+  int rc = b2v_flush(s);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> sub(s->submit_mu);
+  CK(cudaSetDevice(s->device));
+  // one NV12 target per resident frame so that reads AND writes cycle through > L2 of memory
+  std::vector<uint8_t*> outs(n_resident, nullptr);
+  size_t ob = (size_t)s->coded_w * s->coded_h * 3 / 2;
+  for (auto& o : outs) CK(cudaMalloc((void**)&o, ob));
+  for (int i = 0; i < n_resident; i++) launch_csc(csc_params(s, s->resident[i], s->src_w * 4, outs[i]), s->st_enc);   // warm-up
+  CK(cudaStreamSynchronize(s->st_enc));
+  const int n_pairs = per_launch ? iters : 1;
+  std::vector<cudaEvent_t> e0(n_pairs), e1(n_pairs);
+  for (int i = 0; i < n_pairs; i++) { cudaEventCreate(&e0[i]); cudaEventCreate(&e1[i]); }
+  if (!per_launch) cudaEventRecord(e0[0], s->st_enc);
+  for (int i = 0; i < iters; i++) {
+    int k = i % n_resident;
+    if (per_launch) cudaEventRecord(e0[i], s->st_enc);
+    launch_csc(csc_params(s, s->resident[k], s->src_w * 4, outs[k]), s->st_enc);
+    if (per_launch) cudaEventRecord(e1[i], s->st_enc);
+  }
+  if (!per_launch) cudaEventRecord(e1[0], s->st_enc);
+  CK(cudaStreamSynchronize(s->st_enc));
+  double total = 0;
+  for (int i = 0; i < n_pairs; i++) { float ms = 0; cudaEventElapsedTime(&ms, e0[i], e1[i]); total += ms; cudaEventDestroy(e0[i]); cudaEventDestroy(e1[i]); }
+  for (auto o : outs) cudaFree(o);
+  CK(cudaGetLastError());
+  *ms_per_launch = per_launch ? (float)(total / iters) : (float)total / iters;
+  return 0;
 }
 
 }  // namespace
@@ -514,10 +536,8 @@ int b2v_create(const b2v_settings* cfg, b2v_cb cb, void* user, void** out) {
   if (!cfg || !out) return fail(B2V_EINVAL, "null argument");
   int sw = cfg->src_w, sh = cfg->src_h;
   int dw = cfg->dst_w > 0 ? cfg->dst_w : sw, dh = cfg->dst_h > 0 ? cfg->dst_h : sh;
-  if (sw < 16 || sh < 16 || sw > 7680 || sh > 4320 || (sw & 1) || (sh & 1))
-    return fail(B2V_EINVAL, "source size %dx%d unsupported (even, 16..7680 x 16..4320)", sw, sh);
-  if (dw < 16 || dh < 16 || dw > 7680 || dh > 4320 || (dw & 1) || (dh & 1))
-    return fail(B2V_EINVAL, "encoded size %dx%d unsupported", dw, dh);
+  if (!size_supported(sw, sh)) return fail(B2V_EINVAL, "source size %dx%d unsupported (even, 16..7680 x 16..4320)", sw, sh);
+  if (!size_supported(dw, dh)) return fail(B2V_EINVAL, "encoded size %dx%d unsupported", dw, dh);
   int ndev = 0;
   CK(cudaGetDeviceCount(&ndev));
   if (cfg->device < 0 || cfg->device >= ndev) return fail(B2V_EINVAL, "device %d out of range (%d devices)", cfg->device, ndev);
@@ -537,9 +557,6 @@ int b2v_create(const b2v_settings* cfg, b2v_cb cb, void* user, void** out) {
   s->qp_fixed = cfg->crf >= 0 ? cfg->crf : 26;     // 0 is a valid QP; negative = library default
   if (s->qp_fixed > 51) s->qp_fixed = 51;
   s->cb = cb; s->user = user;
-  cudaDeviceProp prop;
-  CK(cudaGetDeviceProperties(&prop, cfg->device));
-  s->sm_count = prop.multiProcessorCount;
   cudaStreamCreateWithFlags(&s->st_copy, cudaStreamNonBlocking);
   // (stream priorities — analysis high, entropy low — were tried and cost 4.5 %: 6520 vs 6830 pictures/s, three runs each)
   cudaStreamCreateWithFlags(&s->st_enc, cudaStreamNonBlocking);
@@ -552,7 +569,7 @@ int b2v_create(const b2v_settings* cfg, b2v_cb cb, void* user, void** out) {
     cudaEventCreateWithFlags(&s->ev_enc[i], cudaEventDisableTiming);
     cudaEventCreateWithFlags(&s->ev_out[i], cudaEventDisableTiming);
   }
-  for (int i = 0; i < kMaxSlots; i++) for (int k = 0; k < 8; k++) cudaEventCreate(&s->ev_t[i][k]);
+  for (int i = 0; i < kMaxSlots; i++) for (int k = 0; k < kTimingEvents; k++) cudaEventCreate(&s->ev_t[i][k]);
   cudaEventCreate(&s->ev_timer[0]); cudaEventCreate(&s->ev_timer[1]);
   if (s->timing && (cfg->flags & B2V_FLAG_DEVICE_TIMER)) cudaMalloc((void**)&s->d_csc_ts, sizeof(unsigned long long) * 2 * kMaxSlots);
   int rc = alloc_geometry(s);
@@ -702,8 +719,7 @@ int b2v_set_resolution(void* h, int32_t sw, int32_t sh, int32_t dw, int32_t dh) 
   if (!s) return fail(B2V_EINVAL, "null handle");
   if (dw <= 0) dw = sw;
   if (dh <= 0) dh = sh;
-  if (sw < 16 || sh < 16 || sw > 7680 || sh > 4320 || (sw & 1) || (sh & 1) || dw < 16 || dh < 16 || dw > 7680 || dh > 4320 || (dw & 1) || (dh & 1))
-    return fail(B2V_EINVAL, "size unsupported");
+  if (!size_supported(sw, sh) || !size_supported(dw, dh)) return fail(B2V_EINVAL, "size unsupported");
   // Submitters are locked out FIRST; then everything in flight drains (the output thread needs `mu`, not `submit_mu`, so it
   // keeps delivering); a producer still holding an acquired slot would be writing into memory about to be freed: refuse.
   std::lock_guard<std::mutex> sub(s->submit_mu);
@@ -792,38 +808,7 @@ int b2v_get_recon(void* h, void* nv12) {
 }
 
 int b2v_bench_csc(void* h, int32_t n_resident, int32_t iters, float* ms_per_launch) {
-  Session* s = (Session*)h;
-  if (!s || n_resident <= 0 || n_resident > (int)s->resident.size() || iters <= 0 || !ms_per_launch) return fail(B2V_EINVAL, "bad argument");
-  int rc = b2v_flush(h);
-  if (rc) return rc;
-  std::lock_guard<std::mutex> sub(s->submit_mu);
-  CK(cudaSetDevice(s->device));
-  // one NV12 target per resident frame so that reads AND writes cycle through > L2 of memory
-  std::vector<uint8_t*> outs(n_resident, nullptr);
-  size_t ob = (size_t)s->coded_w * s->coded_h * 3 / 2;
-  for (auto& o : outs) CK(cudaMalloc((void**)&o, ob));
-  for (int i = 0; i < n_resident; i++) {   // warm-up: one pass over every frame
-    CscParams p = csc_params(s, s->resident[i], s->src_w * 4, outs[i]);
-    launch_csc(p, s->st_enc);
-  }
-  CK(cudaStreamSynchronize(s->st_enc));
-  // each launch is bracketed by its own event pair; the sum excludes host launch gaps
-  std::vector<cudaEvent_t> e0(iters), e1(iters);
-  for (int i = 0; i < iters; i++) { cudaEventCreate(&e0[i]); cudaEventCreate(&e1[i]); }
-  for (int i = 0; i < iters; i++) {
-    int k = i % n_resident;
-    CscParams p = csc_params(s, s->resident[k], s->src_w * 4, outs[k]);
-    cudaEventRecord(e0[i], s->st_enc);
-    launch_csc(p, s->st_enc);
-    cudaEventRecord(e1[i], s->st_enc);
-  }
-  CK(cudaStreamSynchronize(s->st_enc));
-  double total = 0;
-  for (int i = 0; i < iters; i++) { float ms = 0; cudaEventElapsedTime(&ms, e0[i], e1[i]); total += ms; cudaEventDestroy(e0[i]); cudaEventDestroy(e1[i]); }
-  for (auto o : outs) cudaFree(o);
-  CK(cudaGetLastError());
-  *ms_per_launch = (float)(total / iters);
-  return 0;
+  return bench_csc((Session*)h, n_resident, iters, true, ms_per_launch);
 }
 
 int b2v_timer_start(void* h) {
@@ -852,28 +837,7 @@ int b2v_timer_stop(void* h, float* ms) {
 }
 
 int b2v_bench_csc_burst(void* h, int32_t n_resident, int32_t iters, float* ms_per_launch) {
-  Session* s = (Session*)h;
-  if (!s || n_resident <= 0 || n_resident > (int)s->resident.size() || iters <= 0 || !ms_per_launch) return fail(B2V_EINVAL, "bad argument");
-  int rc = b2v_flush(h);
-  if (rc) return rc;
-  std::lock_guard<std::mutex> sub(s->submit_mu);
-  CK(cudaSetDevice(s->device));
-  std::vector<uint8_t*> outs(n_resident, nullptr);
-  size_t ob = (size_t)s->coded_w * s->coded_h * 3 / 2;
-  for (auto& o : outs) CK(cudaMalloc((void**)&o, ob));
-  for (int i = 0; i < n_resident; i++) launch_csc(csc_params(s, s->resident[i], s->src_w * 4, outs[i]), s->st_enc);
-  CK(cudaStreamSynchronize(s->st_enc));
-  cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
-  cudaEventRecord(e0, s->st_enc);
-  for (int i = 0; i < iters; i++) { int k = i % n_resident; launch_csc(csc_params(s, s->resident[k], s->src_w * 4, outs[k]), s->st_enc); }
-  cudaEventRecord(e1, s->st_enc);
-  CK(cudaStreamSynchronize(s->st_enc));
-  float ms = 0; cudaEventElapsedTime(&ms, e0, e1);
-  cudaEventDestroy(e0); cudaEventDestroy(e1);
-  for (auto o : outs) cudaFree(o);
-  CK(cudaGetLastError());
-  *ms_per_launch = ms / iters;
-  return 0;
+  return bench_csc((Session*)h, n_resident, iters, false, ms_per_launch);
 }
 
 }  // extern "C"

@@ -73,8 +73,6 @@ struct FrameCtx {          // everything a kernel needs about the picture being 
   uint8_t* nnz;            // [mbs][32]: 0..15 luma raster, 16..19 Cb, 20..23 Cr
   uint32_t* mb_words;      // [mbs][MB_WORDS]
   uint32_t* mb_nbits;      // [mbs]: bit count | I_PCM flag in bit 30 | skip flag in bit 31
-  long long* mb_off;       // [mbs]: unused (k_slice_build keeps macroblock bit offsets in shared memory)
-  int* mb_run;             // [mbs]: unused (likewise the mb_skip_run preceding each macroblock)
   uint32_t* slice_buf;     // [n_slices][slice_words]
   int slice_words;
   uint32_t* slice_size;    // [n_slices] final NAL bytes (start code + header + EP'd payload)

@@ -30,7 +30,6 @@ struct Encoder {
   uint8_t* i4modes[2] = {nullptr, nullptr};
   int16_t* coef[2] = {nullptr, nullptr};
   uint8_t* nnz[2] = {nullptr, nullptr};
-  long long* mb_off = nullptr; int* mb_run = nullptr;
   void *chunk_agg = nullptr, *chunk_inc = nullptr; int* slice_done = nullptr;   // k_slice_build look-back records (h264_entropy.cu)
   unsigned long long* me_pub = nullptr;   // anchor macroblocks' vectors of the picture being analysed (h264_inter.cu)
   uint32_t *mb_words = nullptr, *mb_nbits = nullptr, *slice_buf = nullptr, *slice_size = nullptr, *slice_rbsp = nullptr;
@@ -165,8 +164,6 @@ int encoder_create(const EncoderConfig* cfg_in, Encoder** out) {
   ECK(cudaMemset(e->me_pub, 0, mbs * sizeof(unsigned long long)));
   ECK(cudaMalloc((void**)&e->mb_words, mbs * MB_WORDS * sizeof(uint32_t)));
   ECK(cudaMalloc((void**)&e->mb_nbits, mbs * sizeof(uint32_t)));
-  ECK(cudaMalloc((void**)&e->mb_off, mbs * sizeof(long long)));
-  ECK(cudaMalloc((void**)&e->mb_run, mbs * sizeof(int)));
   e->slice_words = cfg->slice_rows * e->mbw * MB_WORDS + 64;
   // IDR pictures: slices shorter than a row (same rule as oracle/h264_ref.c auto_seg_cols: about 540 slices, none under 30 macroblocks)
   // (idr_slice_mbs < 0: IDR pictures in slices of slice_rows whole rows, like P pictures — rows of a slice then wait on the row above)
@@ -230,7 +227,7 @@ int encoder_create(const EncoderConfig* cfg_in, Encoder** out) {
 void encoder_destroy(Encoder* e) {
   if (!e) return;
   void* ptrs[] = {e->recon[0], e->recon[1], e->mbinfo[0], e->mbinfo[1], e->coef[0], e->coef[1], e->nnz[0], e->nnz[1], e->mb_words, e->mb_nbits, e->slice_buf,
-                  e->slice_size, e->slice_rbsp, e->slice_bits, e->progress, e->overflow, e->rc, e->param_sets, e->mb_off, e->mb_run, e->i4modes[0],
+                  e->slice_size, e->slice_rbsp, e->slice_bits, e->progress, e->overflow, e->rc, e->param_sets, e->i4modes[0],
                   e->i4modes[1], e->band_fn, e->band_coded, e->me_pub, e->chunk_agg, e->chunk_inc, e->slice_done};
   for (void* p : ptrs) if (p) cudaFree(p);
   for (int b = 0; b < 2; b++) {
@@ -264,7 +261,7 @@ int encoder_encode(Encoder* e, const EncodeFrameParams* p, cudaStream_t st) {
     const int rows_last = e->mbh - (e->n_bands - 1) * e->band_rows;
     f.n_anchor = ((e->mbw + 3) / 4) * ((e->n_bands - 1) * ((e->band_rows + 3) / 4) + (rows_last + 3) / 4);
   }
-  f.mb_words = e->mb_words; f.mb_nbits = e->mb_nbits; f.mb_off = e->mb_off; f.mb_run = e->mb_run;
+  f.mb_words = e->mb_words; f.mb_nbits = e->mb_nbits;
   f.slice_buf = e->slice_buf; f.slice_words = seg ? e->seg_slice_words : e->slice_words; f.slice_size = e->slice_size; f.slice_rbsp = e->slice_rbsp;
   f.slice_bits = e->slice_bits; f.paint_trigger = p->paint_trigger; f.paint_qp = p->paint_qp; f.paint_burst = p->paint_burst; f.progress = e->progress; f.rc = e->rc;
   f.band_rows = e->band_rows; f.n_bands = e->n_bands; f.striped = e->striped; f.param_len_last = e->param_len_last;

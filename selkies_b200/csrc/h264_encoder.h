@@ -15,7 +15,6 @@ struct EncoderConfig {
   int slice_rows;          // macroblock rows per slice
   int stripe_rows;         // macroblock rows per band (multiple of slice_rows); 0 = full-frame
   int idr_slice_mbs;       // IDR pictures: macroblocks per slice inside a row (needs slice_rows == 1); 0 = default rule, < 0 = whole rows
-  int sm_count;
 };
 
 // 64-byte record the pack kernel writes in front of the access unit in HBM; travels to the host
@@ -44,7 +43,7 @@ struct EncodeFrameParams {
   int qp_fixed;
   int paint_trigger, paint_qp, paint_burst;   // paint-over: `paint_burst` pictures at paint_qp after `paint_trigger` all-skipped pictures (0 = off)
   int64_t target_bits;     // per frame, CBR
-  cudaEvent_t* ev;         // null, or 8 timing events: encoder records ev[2..5] after each stage (forces the serial schedule)
+  cudaEvent_t* ev;         // null, or 6 timing events: encoder records ev[2..5] after each stage (forces the serial schedule)
   cudaStream_t st_pack;    // null = everything on `st`; else the entropy coding of this picture (k_cavlc_mb ... k_pack_au) runs here,
                            // overlapping the analysis of the next picture on `st`.  The access unit is complete on st_pack.
   const unsigned long long* csc_ts;   // null, or the CSC launch's device stamps to forward in the AuHeader
