@@ -1,29 +1,10 @@
-// h264_cavlc.cuh — bit sinks and the CAVLC residual-block coder (ITU-T H.264 9.2), shared by the entropy
-// kernels (which write bits) and the analysis kernels (which only SIZE a macroblock to decide I_PCM).
+// h264_cavlc.cuh — the CAVLC residual-block coder (ITU-T H.264 9.2), shared by the entropy kernels (which write bits) and
+// the analysis kernels (which only SIZE a macroblock to decide I_PCM).
 #pragma once
+#include "bitstream.cuh"
 #include "h264_tables.cuh"
 
 namespace b2v {
-
-struct CountSink {
-  int n = 0;
-  __device__ __forceinline__ void put(int len, uint32_t) { n += len; }
-};
-struct SmemSink {           // MSB-first into big-endian u32 words, concurrent writers use atomicOr
-  uint32_t* w; int pos; int cap_bits;
-  __device__ __forceinline__ void put(int len, uint32_t v) {
-    if (len == 0) return;
-    if (pos + len <= cap_bits) {
-      const int wi = pos >> 5, o = pos & 31, space = 32 - o;
-      if (len <= space) atomicOr(&w[wi], v << (space - len));
-      else { atomicOr(&w[wi], v >> (len - space)); atomicOr(&w[wi + 1], v << (32 - (len - space))); }
-    }
-    pos += len;
-  }
-};
-template <class S> __device__ __forceinline__ void put_ue(S& s, uint32_t v) { const int len = 31 - __clz(v + 1); s.put(2 * len + 1, v + 1); }
-template <class S> __device__ __forceinline__ void put_se(S& s, int v) { put_ue(s, v > 0 ? (uint32_t)(2 * v - 1) : (uint32_t)(-2 * v)); }
-__device__ __forceinline__ int ue_len(uint32_t v) { return 2 * (31 - __clz(v + 1)) + 1; }
 
 constexpr int NC_CHROMA_DC = -1;   // coeff_token table for chroma DC
 constexpr int NC_WORST = -2;       // size estimate: the longest coeff_token of the four nC tables

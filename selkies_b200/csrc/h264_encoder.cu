@@ -10,6 +10,7 @@
 
 #include "h264_common.cuh"
 #include <algorithm>
+#include "b2v_internal.h"
 #include "h264_encoder.h"
 #include "h264_kernels.h"
 
@@ -207,7 +208,7 @@ int encoder_create(const EncoderConfig* cfg_in, Encoder** out) {
     std::vector<uint8_t> last = make_param_sets(*cfg, e->mbw, e->mbh - (e->n_bands - 1) * e->band_rows, crop_b);
     e->param_len_last = (int)last.size();
     ps.insert(ps.end(), last.begin(), last.end());
-    e->au_data_off = (int)sizeof(AuHeader) + ((e->n_bands * (int)sizeof(BandEntry) + 16 + 63) & ~63);
+    e->au_data_off = au_data_offset(e->n_bands);
   }
   ECK(cudaMalloc((void**)&e->param_sets, ps.size()));
   ECK(cudaMemcpy(e->param_sets, ps.data(), ps.size(), cudaMemcpyHostToDevice));

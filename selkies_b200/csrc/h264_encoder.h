@@ -17,24 +17,6 @@ struct EncoderConfig {
   int idr_slice_mbs;       // IDR pictures: macroblocks per slice inside a row (needs slice_rows == 1); 0 = default rule, < 0 = whole rows
 };
 
-// 64-byte record the pack kernel writes in front of the access unit in HBM; travels to the host
-// with the first D2H chunk.
-struct AuHeader {
-  int32_t size;            // bytes of Annex-B data following this header
-  int32_t qp;              // slice QP used
-  int32_t is_idr;
-  int32_t n_slices;
-  int64_t total_bits;      // before emulation prevention
-  int32_t next_qp;         // rate controller output for the next frame
-  int32_t overflow;        // non-zero if a macroblock exceeded its scratch budget (must never happen)
-  uint64_t csc_t0, csc_t1;  // %globaltimer stamps of the CSC launch of this picture (0 when timing is off)
-  int32_t pad[4];
-};
-static_assert(sizeof(AuHeader) == 64, "AuHeader must be 64 bytes");
-
-// striped mode: one record per band right after the AuHeader (offsets relative to the first NAL byte)
-struct BandEntry { int32_t off, size, coded, frame_num; };
-
 struct EncodeFrameParams {
   const uint8_t* cur;      // NV12, coded size, device
   uint8_t* au;             // device buffer, encoder_au_capacity() bytes; AuHeader first

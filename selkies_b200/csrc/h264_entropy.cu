@@ -10,13 +10,12 @@
 //                 the slice give every macroblock its bit offset and its mb_skip_run; 8 threads per macroblock shift the bit
 //                 strings into the slice RBSP (atomicOr); the chunk that finishes last counts the slice's emulation-prevention
 //                 bytes; the last block of the picture runs the rate-control step
-//   k_pack_au     one block per slice: prefix over slice sizes, emulation prevention (parallel rule: a 03 is
-//                 inserted before byte i iff byte<=3 and the run of zero bytes before it is even and >=2),
-//                 start codes + NAL headers, AuHeader, band table.
+//   k_pack_au     one block per slice: prefix over slice sizes, emulation prevention (H264Escape; the count in k_slice_build
+//                 and this copy share it, bitstream.cuh), start codes + NAL headers, parameter sets, AuHeader, band table.
 // CPU restatement: oracle/h264_ref.c cavlc_block(), code_slice(), nal_write(), rc_update().
 #include "h264_common.cuh"
 #include "h264_cavlc.cuh"
-#include "h264_encoder.h"
+#include "b2v_internal.h"
 #include "h264_kernels.h"
 
 namespace b2v {
@@ -72,6 +71,21 @@ __device__ __forceinline__ void mb_header_i4(S& h, const FrameCtx& f, const MbIn
   put_ue(h, mi.chroma_mode);
   put_ue(h, cbp_to_codenum_intra[mi.cbp]);
   if (mi.cbp) put_se(h, 0);
+}
+
+// macroblock header of a coded (not P_Skip, not I_PCM) macroblock: I_NxN above; I_16x16: mb_type, intra_chroma_pred_mode,
+// mb_qp_delta; P_L0_16x16: mb_type, mvd_l0, coded_block_pattern (inter me(v) mapping) [, mb_qp_delta]
+template <class S>
+__device__ __forceinline__ void mb_header(S& h, const FrameCtx& f, const MbInfo& mi, int mb, int mbx, int mby, int mvdx, int mvdy,
+                                          int cbp_l, int cbp_c) {
+  if (mi.type == MB_I4) mb_header_i4(h, f, mi, mb, mbx, mby);
+  else if (mi.type == MB_I16) {
+    const int tcode = 1 + mi.i16_mode + 4 * cbp_c + (cbp_l ? 12 : 0);
+    put_ue(h, (uint32_t)(f.idr ? tcode : tcode + 5)); put_ue(h, mi.chroma_mode); put_se(h, 0);
+  } else {
+    put_ue(h, 0); put_se(h, mvdx); put_se(h, mvdy); put_ue(h, cbp_to_codenum_inter[mi.cbp]);
+    if (mi.cbp) put_se(h, 0);
+  }
 }
 
 // ------------------------------------------------------------------------------------------------ k_cavlc_mb
@@ -156,18 +170,7 @@ __global__ void __launch_bounds__(32 * CAVLC_WARPS) k_cavlc_mb(FrameCtx f) {
   CountSink cs;
   if (coded) cavlc_block(cs, lv, maxc, nC);
   int hdr_bits;
-  {
-    CountSink h;
-    if (mi.type == MB_I4) mb_header_i4(h, f, mi, mb, mbx, mby);
-    else if (mi.type == MB_I16) {
-      const int tcode = 1 + mi.i16_mode + 4 * cbp_c + (cbp_l ? 12 : 0);
-      put_ue(h, (uint32_t)(f.idr ? tcode : tcode + 5)); put_ue(h, mi.chroma_mode); put_se(h, 0);
-    } else {
-      put_ue(h, 0); put_se(h, mvdx); put_se(h, mvdy); put_ue(h, cbp_to_codenum_inter[mi.cbp]);
-      if (mi.cbp) put_se(h, 0);
-    }
-    hdr_bits = h.n;
-  }
+  { CountSink h; mb_header(h, f, mi, mb, mbx, mby, mvdx, mvdy, cbp_l, cbp_c); hdr_bits = h.n; }
   int incl = cs.n;
 #pragma unroll
   for (int d = 1; d < 32; d <<= 1) { const int o = __shfl_up_sync(FULL, incl, d); if (lane >= d) incl += o; }
@@ -175,17 +178,7 @@ __global__ void __launch_bounds__(32 * CAVLC_WARPS) k_cavlc_mb(FrameCtx f) {
   const int my_off = hdr_bits + incl - cs.n;
 
   // ---- pass 2: write -----------------------------------------------------------------------------------
-  if (lane == 0) {
-    SmemSink h{words, 0, MB_WORDS * 32};
-    if (mi.type == MB_I4) mb_header_i4(h, f, mi, mb, mbx, mby);
-    else if (mi.type == MB_I16) {
-      const int tcode = 1 + mi.i16_mode + 4 * cbp_c + (cbp_l ? 12 : 0);
-      put_ue(h, (uint32_t)(f.idr ? tcode : tcode + 5)); put_ue(h, mi.chroma_mode); put_se(h, 0);
-    } else {
-      put_ue(h, 0); put_se(h, mvdx); put_se(h, mvdy); put_ue(h, cbp_to_codenum_inter[mi.cbp]);
-      if (mi.cbp) put_se(h, 0);
-    }
-  }
+  if (lane == 0) { SmemSink h{words, 0, MB_WORDS * 32}; mb_header(h, f, mi, mb, mbx, mby, mvdx, mvdy, cbp_l, cbp_c); }
   if (coded) { SmemSink ws{words, my_off, MB_WORDS * 32}; cavlc_block(ws, lv, maxc, nC); }
   __syncwarp();
   int nb = total_bits;
@@ -196,8 +189,11 @@ __global__ void __launch_bounds__(32 * CAVLC_WARPS) k_cavlc_mb(FrameCtx f) {
 }
 
 // ------------------------------------------------------------------------------------------------ slice header (7.3.3)
+// of the slice at geo; first_mb_in_slice and frame_num count within its band (each band is a picture of its own when striped)
 template <class S>
-__device__ __forceinline__ void slice_header(S& s, const FrameCtx& f, int first_mb, int qp, int frame_num) {
+__device__ __forceinline__ void slice_header(S& s, const FrameCtx& f, const SliceGeo& geo, int qp) {
+  const int band = geo.row0 / f.band_rows;
+  const int first_mb = geo.mb0 - band * f.band_rows * f.mbw, frame_num = f.idr ? 0 : f.striped ? f.band_fn[band] : f.frame_num;
   put_ue(s, (uint32_t)first_mb);
   put_ue(s, f.idr ? 7u : 5u);
   put_ue(s, 0);
@@ -209,27 +205,8 @@ __device__ __forceinline__ void slice_header(S& s, const FrameCtx& f, int first_
   put_ue(s, 1);
 }
 
-struct GlobalSink {         // same layout as SmemSink, on the slice's RBSP words in HBM
-  uint32_t* w; long long pos;
-  __device__ __forceinline__ void put(int len, uint32_t v) {
-    if (len == 0) return;
-    const long long wi = pos >> 5; const int o = (int)(pos & 31), space = 32 - o;
-    if (len <= space) atomicOr(&w[wi], v << (space - len));
-    else { atomicOr(&w[wi], v >> (len - space)); atomicOr(&w[wi + 1], v << (32 - (len - space))); }
-    pos += len;
-  }
-};
-
 constexpr int SLICE_THREADS = 256;
-
-__device__ __forceinline__ uint32_t rbsp_byte(const uint32_t* w, long long i) { return (__ldcg(&w[i >> 2]) >> (24 - 8 * (int)(i & 3))) & 255u; }
-
-__device__ __forceinline__ void or_word(uint32_t* out, long long bitpos, uint32_t v) {
-  if (!v) return;
-  const long long wi = bitpos >> 5; const int o = (int)(bitpos & 31);
-  if (o == 0) atomicOr(&out[wi], v);
-  else { atomicOr(&out[wi], v >> o); atomicOr(&out[wi + 1], v << (32 - o)); }
-}
+static_assert(SLICE_THREADS == STUFF_THREADS, "the last chunk of a slice counts its emulation-prevention bytes");
 
 // ---- rate-control / paint-over step, run by the LAST slice-scan block of the picture (thread 0).  The picture's RBSP bit count
 // is known at that point (the byte stream adds emulation prevention, which the controller does not need), so the feedback
@@ -287,33 +264,12 @@ __device__ __forceinline__ void rc_step(const FrameCtx& f, int qp_used, long lon
   rc->fb[f.pic & 1] = n;
 }
 
-// ---- slice_ep_body: one block counts the emulation-prevention bytes slice s needs (7.4.1): a 03 goes in
-// front of byte i iff byte <= 3 and the run of zero bytes before it is even and >= 2.
+// ---- slice_ep_body: one block counts the emulation-prevention bytes slice s needs and publishes its NAL size
 __device__ __forceinline__ void slice_ep_body(const FrameCtx& f, int s) {
   __shared__ int s_red[SLICE_THREADS / 32];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const uint32_t* out = f.slice_buf + (size_t)s * f.slice_words;
   const long long rbsp_bytes = __ldcg(&f.slice_rbsp[s]);
-  int ep = 0;
-  for (long long w0 = (long long)tid * 4; w0 < rbsp_bytes; w0 += SLICE_THREADS * 4) {
-    const uint32_t word = __ldcg(&out[w0 >> 2]);
-#pragma unroll
-    for (int k = 0; k < 4; k++) {
-      const long long i = w0 + k;
-      const uint32_t b = (word >> (24 - 8 * k)) & 255u;
-      if (i < rbsp_bytes && b <= 3u) {
-        int z = 0;
-        while (i - 1 - z >= 0 && rbsp_byte(out, i - 1 - z) == 0u) z++;
-        if (z >= 2 && (z & 1) == 0) ep++;
-      }
-    }
-  }
-  ep = __reduce_add_sync(FULL, ep);
-  if (lane == 0) s_red[warp] = ep;
-  __syncthreads();
-  if (tid == 0) {
-    int t = 0;
-    for (int w = 0; w < SLICE_THREADS / 32; w++) t += s_red[w];
+  const int t = count_escapes<H264Escape>(f.slice_buf + (size_t)s * f.slice_words, rbsp_bytes, s_red);
+  if (threadIdx.x == 0) {
     const SliceGeo geo = slice_geo(f, s);
     const int start_len = (geo.row0 % f.band_rows == 0 && geo.x0 == 0 && !f.idr) ? 4 : 3;     // 4-byte start code on the first NAL of (each band's) access unit
     f.slice_size[s] = (uint32_t)(start_len + 1 + rbsp_bytes + t);
@@ -401,12 +357,7 @@ __global__ void __launch_bounds__(SLICE_THREADS, 8) k_slice_build(FrameCtx f) {
     if (warp == 0) {
       // base state in front of chunk 0: the slice header (every chunk can size it: no waiting for chunk 0)
       long long bits; int trail = 0; bool ok = true;
-      {
-        CountSink h;
-        const int band = geo.row0 / f.band_rows;
-        slice_header(h, f, geo.mb0 - band * f.band_rows * f.mbw, qp, f.idr ? 0 : f.striped ? f.band_fn[band] : f.frame_num);
-        bits = h.n;
-      }
+      { CountSink h; slice_header(h, f, geo, qp); bits = h.n; }
       int start = 0;
       // nearest predecessor whose inclusive state is already there (32 at a time, nearest first)
       for (int hi = k - 1; hi >= 0 && start == 0; hi -= 32) {
@@ -478,11 +429,7 @@ __global__ void __launch_bounds__(SLICE_THREADS, 8) k_slice_build(FrameCtx f) {
       c->bits = s_bits_out; c->trailing = s_trail_out;
       __threadfence();
       *reinterpret_cast<volatile int*>(&c->flag) = tag;
-      if (k == 0) {                              // slice header (the bits it occupies were counted above)
-        GlobalSink g{out, 0};
-        const int band = geo.row0 / f.band_rows;
-        slice_header(g, f, geo.mb0 - band * f.band_rows * f.mbw, qp, f.idr ? 0 : f.striped ? f.band_fn[band] : f.frame_num);
-      }
+      if (k == 0) { GlobalSink g{out, 0}; slice_header(g, f, geo, qp); }     // (the bits it occupies were counted above)
       if (last_chunk) {                          // trailing mb_skip_run, rbsp_trailing_bits
         GlobalSink g{out, s_bits_out};
         const int runt = s_trail_out;
@@ -507,14 +454,9 @@ __global__ void __launch_bounds__(SLICE_THREADS, 8) k_slice_build(FrameCtx f) {
     __threadfence();
     long long bits = 0;
     for (int j = tid; j < f.n_slices; j += SLICE_THREADS) bits += __ldcg(&f.slice_bits[j]);
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) bits += __shfl_xor_sync(FULL, bits, d);
     __syncthreads();
-    if (lane == 0) s_warp_sum[warp] = bits;
-    __syncthreads();
+    const long long t = block_sum<SLICE_THREADS>(bits, s_warp_sum);
     if (tid == 0) {
-      long long t = 0;
-      for (int w = 0; w < SLICE_THREADS / 32; w++) t += s_warp_sum[w];
       f.rc->scan_done = 0;
       rc_step(f, qp, t);
     }
@@ -567,39 +509,31 @@ __global__ void __launch_bounds__(SLICE_THREADS, 8) k_slice_build(FrameCtx f) {
 }
 
 // ------------------------------------------------------------------------------------------------ k_pack_au
-constexpr int PACK_THREADS = 256;
-constexpr int PACK_CH = 16;      // bytes per thread per round
+constexpr int PACK_THREADS = STUFF_THREADS;
 
 __global__ void __launch_bounds__(PACK_THREADS) k_pack_au(FrameCtx f, long long au_cap) {
   __shared__ long long s_base;
+  __shared__ long long s_part[PACK_THREADS / 32];
   __shared__ int s_wsum[PACK_THREADS / 32];
   __shared__ int s_carry;
-  const int s = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int s = blockIdx.x, tid = threadIdx.x;
   // the controller has already moved on to the next picture (rc_step ran in k_slice_build, before this kernel and possibly on another
   // stream): this picture's QP is the one it recorded
   const int qp = f.rc->last_qp;
   // byte offset of this slice's NAL inside the access unit
   long long part = 0;
   for (int j = tid; j < s; j += PACK_THREADS) part += f.slice_size[j];
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) part += __shfl_xor_sync(FULL, part, d);
-  __shared__ long long s_part[PACK_THREADS / 32];
-  if (lane == 0) s_part[warp] = part;
-  __syncthreads();
+  part = block_sum<PACK_THREADS>(part, s_part);
   const SliceGeo geo = slice_geo(f, s);
   const int row0 = geo.row0, band = row0 / f.band_rows;
   const bool band_first = row0 == band * f.band_rows && geo.x0 == 0;      // this slice opens its band's access unit
   const int plen = (f.striped && band == f.n_bands - 1) ? f.param_len_last : f.param_len;
-  if (tid == 0) {
-    long long t = f.idr ? (long long)band * f.param_len + plen : 0;       // parameter sets of bands 0..band precede this NAL
-    for (int w = 0; w < PACK_THREADS / 32; w++) t += s_part[w];
-    s_base = t; s_carry = 0;
-  }
+  if (tid == 0) s_base = part + (f.idr ? (long long)band * f.param_len + plen : 0);     // parameter sets of bands 0..band precede this NAL
   __syncthreads();
   uint8_t* au = f.au + f.au_data_off;
   const long long cap = au_cap - (long long)f.au_data_off;
   const long long base = s_base;
-  const uint32_t* in = f.slice_buf + (size_t)s * f.slice_words;
+  uint32_t* rbsp = f.slice_buf + (size_t)s * f.slice_words;
   const long long n = f.slice_rbsp[s];
   const int start_len = (band_first && !f.idr) ? 4 : 3;
   if (tid == 0 && base + start_len + 1 <= cap) {
@@ -609,50 +543,8 @@ __global__ void __launch_bounds__(PACK_THREADS) k_pack_au(FrameCtx f, long long 
     au[o++] = (uint8_t)(((f.idr ? 3 : 2) << 5) | (f.idr ? 5 : 1));
   }
   const long long out0 = base + start_len + 1;
-  for (long long cb = 0; cb < n; cb += (long long)PACK_THREADS * PACK_CH) {
-    const long long i0 = cb + (long long)tid * PACK_CH;
-    uint32_t bytes[PACK_CH]; uint32_t epmask = 0; int cnt = 0;
-    if (i0 < n) {
-      int z = 0;                                   // zero run in front of the chunk
-      while (i0 - 1 - z >= 0 && rbsp_byte(in, i0 - 1 - z) == 0u) z++;
-#pragma unroll
-      for (int k = 0; k < PACK_CH; k++) {
-        const long long i = i0 + k;
-        const uint32_t b = i < n ? rbsp_byte(in, i) : 0xffu;
-        bytes[k] = b;
-        if (i < n && b <= 3u && z >= 2 && (z & 1) == 0) { epmask |= 1u << k; cnt++; }
-        z = b == 0u ? z + 1 : 0;
-      }
-    }
-    int incl = cnt;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) { const int o = __shfl_up_sync(FULL, incl, d); if (lane >= d) incl += o; }
-    if (lane == 31) s_wsum[warp] = incl;
-    __syncthreads();
-    int before = s_carry;
-    for (int w = 0; w < warp; w++) before += s_wsum[w];
-    before += incl - cnt;
-    if (i0 < n) {
-      long long o = out0 + i0 + before;
-#pragma unroll
-      for (int k = 0; k < PACK_CH; k++) {
-        if (i0 + k < n) {
-          if ((epmask >> k) & 1u) { if (o < cap) au[o] = 3; o++; }
-          if (o < cap) au[o] = (uint8_t)bytes[k];
-          o++;
-        }
-      }
-    }
-    __syncthreads();
-    if (tid == 0) { int t = s_carry; for (int w = 0; w < PACK_THREADS / 32; w++) t += s_wsum[w]; s_carry = t; }
-    __syncthreads();
-  }
-  // self-clean the slice scratch for the next picture (k_slice_bits builds the RBSP with atomicOr)
-  {
-    uint32_t* w = f.slice_buf + (size_t)s * f.slice_words;
-    const long long nw = min((long long)f.slice_words, (n >> 2) + 2);
-    for (long long i = tid; i < nw; i += PACK_THREADS) w[i] = 0;
-  }
+  stuff_copy<H264Escape>(rbsp, n, au + out0, cap - out0, s_wsum, s_carry);
+  clear_bits<PACK_THREADS>(rbsp, n, f.slice_words);
   if (band_first) {
     if (f.idr && base <= cap) {
       const uint8_t* ps = f.param_sets + ((f.striped && band == f.n_bands - 1) ? f.param_len : 0);

@@ -13,13 +13,16 @@
 //   k_jpeg_size   one thread per block: DC difference against the previous block of its component, exact Huffman size
 //   k_jpeg_scan   one block per stripe: prefix sum -> bit offset of every block, stripe size
 //   k_jpeg_write  one thread per block: Huffman codes shifted into the stripe's bit string (atomicOr)
-//   k_jpeg_pack   one block per stripe: FF byte stuffing (prefix sum over the FF count), JFIF header, EOI, stripe table
+//   k_jpeg_ff     one block per stripe: pad the last byte with 1-bits, count the FF bytes -> size of the stripe's file
+//   k_jpeg_pack   one block per stripe: JFIF header, FF byte stuffing, EOI, stripe table
+// The bit sinks, the stuffing rule (JpegEscape) and its count and copy are shared with the H.264 back end (bitstream.cuh).
 // CPU restatement (byte-identical to libjpeg-turbo in its single-component mode): oracle/jpeg_ref.c.
 #include <cstdio>
 #include <cstring>
 #include <vector>
 
-#include "h264_encoder.h"     // AuHeader, BandEntry: the JPEG mode reuses the access-unit container of the striped H.264 mode
+#include "b2v_internal.h"     // AuHeader, BandEntry: the JPEG mode uses the access-unit container of the striped H.264 mode
+#include "bitstream.cuh"
 #include "jpeg.h"
 
 namespace b2v {
@@ -112,7 +115,7 @@ size_t make_header(uint8_t* o, int w, int h, int quality, int* h_off) {
 }
 
 constexpr int JPEG_BLOCK_WORDS = 80;           // per-8x8-block share of the stripe bit string: 2560 bits (worst case 63 x 26 + 20 < 1700)
-constexpr int JT = 256;
+constexpr int JT = STUFF_THREADS;
 
 struct JpegCtx {
   int cw, ch, w, h;                 // coded (multiple of 16) and visible size
@@ -241,18 +244,7 @@ __device__ __forceinline__ int prev_block(const JpegCtx& c, int b, int mx, int m
 }
 __device__ __forceinline__ int bitlen_dev(int v) { return 32 - __clz(v); }
 
-struct JCount { int n; __device__ __forceinline__ void put(int len, uint32_t) { n += len; } };
-struct JWrite {
-  uint32_t* w; long long pos;
-  __device__ __forceinline__ void put(int len, uint32_t v) {
-    if (len == 0) return;
-    v &= len >= 32 ? 0xffffffffu : ((1u << len) - 1u);
-    const long long wi = pos >> 5; const int o = (int)(pos & 31), space = 32 - o;
-    if (len <= space) atomicOr(&w[wi], v << (space - len));
-    else { atomicOr(&w[wi], v >> (len - space)); atomicOr(&w[wi + 1], v << (32 - (len - space))); }
-    pos += len;
-  }
-};
+// the magnitude bits of a coefficient: the low nb bits of t (negative t: of t - 1); the Huffman codes fit their lengths already
 template <class S>
 __device__ __forceinline__ void code_block(S& s, const int16_t* lv, int pred_dc, int chroma) {
   int t = (int)lv[0] - pred_dc, t2 = t;
@@ -260,7 +252,7 @@ __device__ __forceinline__ void code_block(S& s, const int16_t* lv, int pred_dc,
   int nb = bitlen_dev(t);
   uint32_t e = c_dc[chroma][nb];
   s.put((int)(e >> 16), e & 0xffffu);
-  s.put(nb, (uint32_t)t2);
+  s.put(nb, (uint32_t)t2 & ((1u << nb) - 1u));
   int r = 0;
   for (int k = 1; k < 64; k++) {
     t = lv[k];
@@ -271,7 +263,7 @@ __device__ __forceinline__ void code_block(S& s, const int16_t* lv, int pred_dc,
     nb = bitlen_dev(t);
     e = c_ac[chroma][(r << 4) + nb];
     s.put((int)(e >> 16), e & 0xffffu);
-    s.put(nb, (uint32_t)t2);
+    s.put(nb, (uint32_t)t2 & ((1u << nb) - 1u));
     r = 0;
   }
   if (r > 0) { e = c_ac[chroma][0]; s.put((int)(e >> 16), e & 0xffffu); }
@@ -288,67 +280,55 @@ __global__ void __launch_bounds__(128) k_jpeg_code(JpegCtx c) {
   const int16_t* lv = c.lev + (size_t)b * 64;
   const int pb = prev_block(c, b, mx, my, k);
   const int pred = pb < 0 ? 0 : (int)c.lev[(size_t)pb * 64];
-  if (WRITE) { JWrite w{c.sbuf + (size_t)s * c.stripe_words, c.off[b]}; code_block(w, lv, pred, k >= 4); }
-  else { JCount n{0}; code_block(n, lv, pred, k >= 4); c.bits[b] = (uint32_t)n.n; }
+  if (WRITE) { GlobalSink w{c.sbuf + (size_t)s * c.stripe_words, c.off[b]}; code_block(w, lv, pred, k >= 4); }
+  else { CountSink n; code_block(n, lv, pred, k >= 4); c.bits[b] = (uint32_t)n.n; }
 }
 
 // ---- scan: block per stripe, prefix sum of the block sizes ---------------------------------------------------------------------
 __global__ void __launch_bounds__(JT) k_jpeg_scan(JpegCtx c) {
   __shared__ long long s_w[JT / 32];
   __shared__ long long s_carry;
-  const int s = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int s = blockIdx.x, tid = threadIdx.x;
   const int my0 = s * c.stripe_rows, my1 = min(c.mcu_h, my0 + c.stripe_rows);
   const int b0 = my0 * c.mcu_w * 6, nb = (my1 - my0) * c.mcu_w * 6;
   if (tid == 0) s_carry = 0;
   __syncthreads();
   for (int base = 0; base < nb; base += JT) {
     const int i = base + tid;
-    const long long v = i < nb ? (long long)c.bits[b0 + i] : 0;
-    long long incl = v;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) { const long long o = __shfl_up_sync(0xffffffffu, incl, d); if (lane >= d) incl += o; }
-    if (lane == 31) s_w[warp] = incl;
-    __syncthreads();
-    long long pre = s_carry;
-    for (int w = 0; w < warp; w++) pre += s_w[w];
-    if (i < nb) c.off[b0 + i] = pre + incl - v;
-    __syncthreads();
-    if (tid == JT - 1) s_carry = pre + incl;
-    __syncthreads();
+    const long long off = block_scan<JT>(i < nb ? (long long)c.bits[b0 + i] : 0LL, s_w, s_carry);
+    if (i < nb) c.off[b0 + i] = off;
   }
   if (tid == 0) c.sbits[s] = s_carry;
 }
-
-__device__ __forceinline__ uint32_t sbyte(const uint32_t* w, long long i) { return (__ldcg(&w[i >> 2]) >> (24 - 8 * (int)(i & 3))) & 255u; }
 
 // ---- ff count: block per stripe.  Pads the last byte with 1-bits, counts the FF bytes (each gets a 00 stuffed behind it) and
 // publishes the size of the stripe's file ------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(JT) k_jpeg_ff(JpegCtx c) {
   __shared__ int s_w[JT / 32];
-  const int s = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int s = blockIdx.x, tid = threadIdx.x;
   if (!(c.s_flags[s] & 1)) { if (tid == 0) c.ssize[s] = 0; return; }
   uint32_t* w = c.sbuf + (size_t)s * c.stripe_words;
   const long long bits = c.sbits[s], nbytes = (bits + 7) >> 3;
   if (tid == 0 && (bits & 7)) { const int padn = 8 - (int)(bits & 7); atomicOr(&w[bits >> 5], ((1u << padn) - 1u) << (32 - (int)(bits & 31) - padn)); __threadfence(); }
   __syncthreads();
-  int cnt = 0;
-  for (long long i = tid; i < nbytes; i += JT) cnt += sbyte(w, i) == 255u;
-  cnt = __reduce_add_sync(0xffffffffu, cnt);
-  if (lane == 0) s_w[warp] = cnt;
-  __syncthreads();
-  if (tid == 0) { int t = 0; for (int k = 0; k < JT / 32; k++) t += s_w[k]; c.ssize[s] = (uint32_t)(c.hdr_len + nbytes + t + 2); }
+  const int ff = count_escapes<JpegEscape>(w, nbytes, s_w);
+  if (tid == 0) c.ssize[s] = (uint32_t)(c.hdr_len + nbytes + ff + 2);
 }
 
 // ---- pack: block per stripe.  header | stuffed scan bytes | EOI, stripes back to back; stripe table entry; AuHeader ------------------
 __global__ void __launch_bounds__(JT) k_jpeg_pack(JpegCtx c) {
   __shared__ int s_w[JT / 32];
   __shared__ int s_carry;
+  __shared__ long long s_part[JT / 32];
   __shared__ long long s_base;
-  const int s = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int s = blockIdx.x, tid = threadIdx.x;
   const int fl = c.s_flags[s];
   uint8_t* au = c.au + c.au_data_off;
   const long long cap = c.au_cap - c.au_data_off;
-  if (tid == 0) { long long t = 0; for (int j = 0; j < s; j++) t += c.ssize[j]; s_base = t; s_carry = 0; }
+  long long part = 0;                                      // byte offset of this stripe's file: the sizes of the stripes before it
+  for (int j = tid; j < s; j += JT) part += c.ssize[j];
+  part = block_sum<JT>(part, s_part);
+  if (tid == 0) s_base = part;
   __syncthreads();
   const long long slot = s_base;
   BandEntry* be = reinterpret_cast<BandEntry*>(c.au + sizeof(AuHeader)) + s;
@@ -372,31 +352,10 @@ __global__ void __launch_bounds__(JT) k_jpeg_pack(JpegCtx c) {
     au[slot + c.hdr_h_off] = (uint8_t)(hh >> 8); au[slot + c.hdr_h_off + 1] = (uint8_t)hh;
   }
   const long long out0 = slot + c.hdr_len;
-  constexpr int CH = 16;
-  for (long long cb = 0; cb < nbytes; cb += (long long)JT * CH) {
-    const long long i0 = cb + (long long)tid * CH;
-    uint32_t by[CH]; int cnt = 0;
-#pragma unroll
-    for (int k = 0; k < CH; k++) { by[k] = i0 + k < nbytes ? sbyte(w, i0 + k) : 0u; cnt += by[k] == 255u; }
-    int incl = cnt;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) { const int o = __shfl_up_sync(0xffffffffu, incl, d); if (lane >= d) incl += o; }
-    if (lane == 31) s_w[warp] = incl;
-    __syncthreads();
-    int before = s_carry;
-    for (int ww = 0; ww < warp; ww++) before += s_w[ww];
-    before += incl - cnt;
-    long long o = out0 + i0 + before;
-#pragma unroll
-    for (int k = 0; k < CH; k++) if (i0 + k < nbytes) { if (o < cap) au[o] = (uint8_t)by[k]; o++; if (by[k] == 255u) { if (o < cap) au[o] = 0; o++; } }
-    __syncthreads();
-    if (tid == 0) { int t = s_carry; for (int ww = 0; ww < JT / 32; ww++) t += s_w[ww]; s_carry = t; }
-    __syncthreads();
-  }
-  // self-clean the bit string for the next picture
-  for (long long i = tid; i < min(c.stripe_words, (nbytes >> 2) + 2); i += JT) w[i] = 0;
+  const int ff = stuff_copy<JpegEscape>(w, nbytes, au + out0, cap - out0, s_w, s_carry);
+  clear_bits<JT>(w, nbytes, c.stripe_words);
   if (tid == 0) {
-    const long long end = out0 + nbytes + s_carry;
+    const long long end = out0 + nbytes + ff;
     if (end + 2 <= cap) { au[end] = 0xFF; au[end + 1] = 0xD9; }
     be->off = (int32_t)slot; be->size = (int32_t)(end + 2 - slot); be->coded = 1; be->frame_num = (fl >> 1) & 1;
   }
@@ -457,7 +416,7 @@ int jpeg_create(const JpegConfig* cfg, JpegEncoder** out) {
   JCK(cudaMalloc((void**)&e->s_static, e->n_stripes * sizeof(int))); JCK(cudaMemset(e->s_static, 0, e->n_stripes * sizeof(int)));
   JCK(cudaMalloc((void**)&e->s_flags, e->n_stripes * sizeof(int)));
   JCK(cudaMalloc((void**)&e->ssize, e->n_stripes * sizeof(uint32_t)));
-  e->au_data_off = (int)sizeof(AuHeader) + ((e->n_stripes * (int)sizeof(BandEntry) + 16 + 63) & ~63);
+  e->au_data_off = au_data_offset(e->n_stripes);
   // output capacity: 16 bits per pixel-equivalent (128 bytes per 8x8 block) — above anything quality <= 100 produces on real content;
   // a picture that would not fit is reported (AuHeader.overflow) and fails the session loudly instead of being truncated silently
   e->au_cap = (size_t)e->au_data_off + (size_t)e->n_stripes * (e->hdr_len + 2) + blocks * 128 + 4096;
